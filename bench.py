@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the hot path (BASELINE.json: "G1 MSM 2^24 ms; NTT 2^24 ms").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -18,6 +18,14 @@ baseline: the arkworks-0.3.0 algorithm restated in C++ (oracle/cpp), timed on th
 
 `--impl reference` times that CPU restatement (arkworks itself cannot be built: no Rust toolchain,
 crates not vendored) with all host threads on a bounded sample and prints the same JSON line.
+
+`--dump-outputs DIR` writes, after the run, what the last timed step returned (rank 0), as float64 .npy
+files holding 32-bit words (exact) of arkworks' u64 limbs, so that two builds can be compared output for
+output on the same seeded inputs:
+  msm_result_xy.npy        (2, 2*L64) the affine MSM result x, y (Montgomery limbs as u32 words)
+  msm_result_infinity.npy  (1,)       1.0 if the result is the point at infinity
+  ntt_sample_index.npy     (S,)       sorted rows of the 2^LOG_N NTT output, a fixed seeded sample
+  ntt_sample_output.npy    (S, 8)     those rows (Fr element, Montgomery, as u32 words)   [not with --skip-ntt]
 """
 from __future__ import annotations
 
@@ -220,7 +228,13 @@ def main():
     ap.add_argument("--skip-proxy", action="store_true", help="skip the Groth16 proof proxy leg")
     ap.add_argument("--skip-precompute", action="store_true", help="skip the precomputed-bases MSM leg")
     ap.add_argument("--skip-single-process", action="store_true", help="skip the one-process-N-GPUs leg (N > 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -342,6 +356,10 @@ def main():
 
     # ---- correctness of what was timed: known-discrete-log identity (exact big-int check on rank 0)
     final = (d_final if world > 1 else d_rec).cpu().numpy().view(np.uint64)
+    dumps = {}      # --dump-outputs: name -> float64 array of the last timed step's outputs (u64 limbs as exact u32 words)
+    if args.dump_outputs:
+        dumps["msm_result_xy"] = final[:W2].view(np.uint32).astype(np.float64).reshape(2, -1)
+        dumps["msm_result_infinity"] = final[W2:].astype(np.float64)
     ok = None
     if rank == 0:
         from oracle.py import exact
@@ -491,7 +509,13 @@ def main():
         def step_ntt():
             _lib.check(L.zkm_ntt_device(CURVE_ID, ctypes.c_void_p(x.data_ptr()), ctypes.c_void_p(y.data_ptr()), LOG_N,
                                         0, 0, sp))
-        ms_ntt, _ = timed(step_ntt, max(args.steps, 5), 3)
+        ms_ntt, _ = timed(step_ntt, args.steps, 3)
+        if args.dump_outputs:
+            rows = np.sort(np.random.Generator(np.random.PCG64(0x5EED2000 + LOG_N)).choice(n_ntt, min(n_ntt, 1 << 16),
+                                                                                          replace=False))
+            dumps["ntt_sample_index"] = rows.astype(np.float64)
+            dumps["ntt_sample_output"] = (y[torch.from_numpy(rows).to(dev)].cpu().numpy().view(np.uint32)
+                                          .astype(np.float64))
         peaks = read_peaks()
         hbm = peaks["hbm_gbs"] if peaks and "hbm_gbs" in peaks else 6650.0
         gbs = 64.0 * n_ntt / (ms_ntt * 1e-3) / 1e9
@@ -647,6 +671,10 @@ def main():
             "single_process_multi_gpu": single,
         }
         line.update(extra)
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -1,9 +1,12 @@
 """bench.py's output contract, checked on CPU through the reference arm (the only arm that runs without a GPU):
-stdout carries exactly ONE JSON line with the keys the driver reads; the CPU arm describes its bounded sample."""
+stdout carries exactly ONE JSON line with the keys its readers rely on; the CPU arm describes its bounded sample.
+On the GPU: what --dump-outputs writes."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -44,3 +47,48 @@ def test_non_zero_ranks_of_the_reference_arm_stay_silent():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
                        capture_output=True, text=True, timeout=120, env=env, cwd=ROOT)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_bench_rejects_arguments_it_cannot_honour(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra,
+                           capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert r.returncode == 2 and r.stdout.strip() == "", (extra, r.stdout, r.stderr[-2000:])
+    assert not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step_and_repeat_exactly(tmp_path):
+    """--dump-outputs: float64 files of exact u32 words, within 64 MB, equal to the CPU oracle on the bench's seeded
+    inputs, and identical from one run to the next."""
+    import numpy as np
+    from oracle import capi
+    log_n = 18
+    env = dict(os.environ, ZKM_BENCH_LOG_N=str(log_n))
+    dumps = []
+    for run in ("a", "b"):
+        out = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", "1",
+                            "--skip-cpu", "--skip-proxy", "--skip-precompute", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, env=env, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-3000:]
+        j = json.loads(r.stdout.strip().splitlines()[-1])
+        assert j["steps"] == 2 and j["config"]["result_ok"] is True
+        files = sorted(p.name for p in out.iterdir())
+        assert files == ["msm_result_infinity.npy", "msm_result_xy.npy", "ntt_sample_index.npy", "ntt_sample_output.npy"]
+        assert sum(p.stat().st_size for p in out.iterdir()) <= 64 << 20
+        d = {f[:-4]: np.load(out / f) for f in files}
+        for a in d.values():
+            assert a.dtype == np.float64 and np.all(a == np.floor(a)) and a.min() >= 0 and a.max() < 2.0 ** 32
+        dumps.append(d)
+    a, b = dumps
+    assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) for k in a)
+    words = lambda u64: u64.view(np.uint32).astype(np.float64)
+    n = 1 << log_n
+    want_xy, want_inf = capi.msm(0, 1, capi.progression(0, 1, 0x1234567, 0x89ABCDE, n),
+                                 capi.random_scalars(0, n, seed=0x5EED0000 + log_n))
+    assert np.array_equal(a["msm_result_xy"].ravel(), words(want_xy)) and a["msm_result_infinity"].tolist() == [float(want_inf)]
+    rows = a["ntt_sample_index"].astype(np.int64)
+    assert len(rows) == 1 << 16 and np.all(np.diff(rows) > 0) and rows[-1] < n
+    want_ntt = capi.ntt(0, capi.random_field_elements(0, n, seed=0x5EED1000 + log_n))
+    assert np.array_equal(a["ntt_sample_output"], words(np.ascontiguousarray(want_ntt[rows])))

@@ -5,6 +5,7 @@ Test vehicle only -- nothing in the shipped library is built with ZKM_HOST_EMU."
 import ctypes
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -168,4 +169,4 @@ def test_xyzz_group_law_with_exceptional_cases(emu, curve, g):
 
 def test_constants_header_is_up_to_date():
     root = os.path.dirname(HERE)
-    assert subprocess.call(["python", os.path.join(root, "tools", "gen_constants.py"), "--check"]) == 0
+    assert subprocess.call([sys.executable, os.path.join(root, "tools", "gen_constants.py"), "--check"]) == 0
