@@ -149,6 +149,29 @@ int32_t zkm_kzg_open(uint64_t handle_g, uint64_t handle_gamma_g, const uint64_t*
                      const uint64_t* blinding_coeffs, size_t nb, const uint64_t* point, uint64_t* out_w_xy,
                      uint8_t* out_w_inf, uint64_t* out_random_v);
 
+/* ---- fixed-base batch scalar multiplication -------------------------------------------------------
+ * Replaces ark_ec::msm::FixedBaseMSM::{get_window_table, multi_scalar_mul} (ark-ec 0.3.0 src/msm/fixed_base.rs)
+ * + batch_normalization_into_affine: the queries of Groth16::circuit_specific_setup (ark-groth16 0.3.0
+ * src/generator.rs) and the powers of KZG10::setup (ark-poly-commit 0.3.0 src/kzg10/mod.rs).
+ * out[i] = scalars[i] * base for i < n, as n normalised affine records (2 * W words, Montgomery) in out_xy plus one
+ * infinity byte each in out_inf; a zero product is arkworks' zero (x = 0, y = 1, flag 1).
+ * scalars: n Montgomery Fr elements (S64 words each), as upstream takes &[G::ScalarField]; base: ONE affine record
+ * (HOST pointer, 2 * W words) and its infinity flag.  A base at infinity gives every output at infinity.
+ * The window width is chosen from n inside the library.  n = 0 succeeds and writes nothing; a null pointer where
+ * n > 0, or an unknown curve or group, gives ZKM_ERR_ARG.
+ * zkm_fixed_base_msm: scalars and outputs are HOST pointers; returns when the outputs are written.  An element
+ * >= r fails with ZKM_ERR_SCALAR_RANGE (checked on the device, read back with the outputs). */
+int32_t zkm_fixed_base_msm(int32_t curve, int32_t group, const uint64_t* base_xy, uint8_t base_inf,
+                           const uint64_t* scalars, size_t n, uint64_t* out_xy, uint8_t* out_inf);
+/* Device-resident form: d_scalars, d_out_xy and d_out_inf are DEVICE pointers (16-byte aligned, see above; the call
+ * runs on the device that owns d_out_xy), base_xy stays a HOST pointer (passed to the kernels by value: nothing is
+ * copied, the call never waits for the host).  A fixed sequence of kernel launches on `stream`, no device read-back.
+ * Elements >= r are NOT checked (like zkm_fr_into_repr_device).  The outputs are in the format of
+ * zkm_bases_register_device: a proving key or SRS built here can be registered without a host round trip. */
+int32_t zkm_fixed_base_msm_device(int32_t curve, int32_t group, const uint64_t* base_xy, uint8_t base_inf,
+                                  const uint64_t* d_scalars, size_t n, uint64_t* d_out_xy, uint8_t* d_out_inf,
+                                  void* stream);
+
 /* ---- radix-2 NTT ------------------------------------------------------------------------------
  * Replaces ark_poly::Radix2EvaluationDomain::{fft_in_place, ifft_in_place, coset_fft_in_place,
  * coset_ifft_in_place} (ark-poly 0.3.0 src/domain/radix2/{mod,fft}.rs, src/domain/mod.rs) on the

@@ -5,6 +5,7 @@
 // (same names, argument meaning and error behaviour); INTEGRATION.md shows the equivalent Rust shim.
 //
 //   zkm::VariableBaseMSM::multi_scalar_mul(bases, scalars)      ark-ec 0.3.0 src/msm/variable_base.rs
+//   zkm::FixedBaseMSM::multi_scalar_mul(base, scalars)          ark-ec 0.3.0 src/msm/fixed_base.rs
 //   zkm::Radix2EvaluationDomain<Curve>::new_(n) / fft / ifft / coset_fft / coset_ifft (+ _in_place)
 //                                                               ark-poly 0.3.0 src/domain/radix2/mod.rs
 //   zkm::witness_map(domain, a, b, c)                           ark-groth16 0.3.0 src/r1cs_to_qap.rs
@@ -186,6 +187,30 @@ struct VariableBaseMSM {
                                 : zkm_msm_g2(Curve::ID, xy.data(), inf.data(), sc, size, out.data(), &out_inf);
         check(rc, "zkm_msm");
         return detail::unpack<Curve, GROUP>(out, out_inf);
+    }
+};
+
+struct FixedBaseMSM {
+    // ark_ec::msm::FixedBaseMSM::{get_window_table, multi_scalar_mul} + batch_normalization_into_affine: scalars[i] * base
+    // for every Montgomery Fr element (the window width is the library's choice)
+    template <class Curve, int GROUP>
+    static std::vector<GroupAffine<Curve, GROUP>> multi_scalar_mul(const GroupAffine<Curve, GROUP>& base,
+                                                                   const std::vector<typename Curve::Fr>& scalars) {
+        typedef typename GroupAffine<Curve, GROUP>::Coord Coord;
+        constexpr size_t W = sizeof(Coord) / 8;
+        std::vector<uint64_t> b, xy(scalars.size() * 2 * W);
+        std::vector<uint8_t> binf, inf(scalars.size());
+        detail::pack<Curve, GROUP>(std::vector<GroupAffine<Curve, GROUP>>{base}, 1, b, binf);
+        check(zkm_fixed_base_msm(Curve::ID, GROUP, b.data(), binf[0], reinterpret_cast<const uint64_t*>(scalars.data()),
+                                 scalars.size(), xy.data(), inf.data()),
+              "zkm_fixed_base_msm");
+        std::vector<GroupAffine<Curve, GROUP>> out(scalars.size());
+        for (size_t i = 0; i < scalars.size(); i++) {
+            std::memcpy(&out[i].x, &xy[i * 2 * W], sizeof(Coord));
+            std::memcpy(&out[i].y, &xy[i * 2 * W + W], sizeof(Coord));
+            out[i].infinity = inf[i] != 0;
+        }
+        return out;
     }
 };
 

@@ -31,6 +31,10 @@ extern "C" {
                       out_xy: *mut u64, out_inf: *mut u8) -> i32;
     pub fn zkm_msm_g2(curve: i32, bases_xy: *const u64, infinity: *const u8, scalars: *const u64, n: usize,
                       out_xy: *mut u64, out_inf: *mut u8) -> i32;
+    pub fn zkm_fixed_base_msm(curve: i32, group: i32, base_xy: *const u64, base_inf: u8, scalars: *const u64, n: usize,
+                              out_xy: *mut u64, out_inf: *mut u8) -> i32;
+    pub fn zkm_fixed_base_msm_device(curve: i32, group: i32, base_xy: *const u64, base_inf: u8, d_scalars: *const u64, n: usize,
+                                     d_out_xy: *mut u64, d_out_inf: *mut u8, stream: *mut c_void) -> i32;
     pub fn zkm_bases_register(curve: i32, group: i32, bases_xy: *const u64, infinity: *const u8, n: usize,
                               handle_out: *mut u64) -> i32;
     pub fn zkm_bases_release(handle: u64) -> i32;

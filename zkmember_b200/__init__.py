@@ -3,7 +3,7 @@
 Only the hot path lives here: `csrc/` (hand-written CUDA for sm_100a + the C ABI of
 include/zkm_b200.h) and the host-side mirrors of the two arkworks interfaces it replaces:
 
-    from zkmember_b200 import VariableBaseMSM, Radix2EvaluationDomain
+    from zkmember_b200 import VariableBaseMSM, FixedBaseMSM, Radix2EvaluationDomain
 """
 import os as _os
 
@@ -14,10 +14,10 @@ import os as _os
 _os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 from ._lib import ZkmError, DomainError, init, shutdown, set_option, launch_count, load  # noqa: F401
-from .msm import VariableBaseMSM, RegisteredBases, AffinePoint, msm_window_bits  # noqa: F401
+from .msm import VariableBaseMSM, FixedBaseMSM, RegisteredBases, AffinePoint, msm_window_bits  # noqa: F401
 from .domain import Radix2EvaluationDomain, GeneralEvaluationDomain  # noqa: F401
 
 __all__ = [
-    "VariableBaseMSM", "RegisteredBases", "AffinePoint", "Radix2EvaluationDomain", "GeneralEvaluationDomain",
+    "VariableBaseMSM", "FixedBaseMSM", "RegisteredBases", "AffinePoint", "Radix2EvaluationDomain", "GeneralEvaluationDomain",
     "ZkmError", "DomainError", "init", "shutdown", "set_option", "launch_count", "load", "msm_window_bits",
 ]

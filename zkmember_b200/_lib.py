@@ -33,6 +33,7 @@ SYMBOLS = [
     "zkm_msm_window_bits", "zkm_testgen_progression_device", "zkm_profile_last_msm", "zkm_witness_map", "zkm_witness_map_device", "zkm_fr_into_repr_device", "zkm_kzg_commit", "zkm_msm_batch_registered_device",
     "zkm_init_mask", "zkm_init_devices", "zkm_initialised_devices", "zkm_bases_register_ex", "zkm_kzg_commit_batch",
     "zkm_kzg_commit_hiding", "zkm_kzg_open", "zkm_profile_last_msm_counts", "zkm_msm_cache_clear", "zkm_msm_cache_stats",
+    "zkm_fixed_base_msm", "zkm_fixed_base_msm_device",
 ]
 
 # zkm_bases_register_ex flags (include/zkm_b200.h)
@@ -106,6 +107,8 @@ def load():
     L.zkm_launch_count.restype = u64
     L.zkm_msm_window_bits.argtypes = [i32, i32, sz]
     L.zkm_testgen_progression_device.argtypes = [i32, i32, u64, u64, sz, u64p, vp]
+    L.zkm_fixed_base_msm.argtypes = [i32, i32, u64p, ctypes.c_uint8, u64p, sz, u64p, u8p]
+    L.zkm_fixed_base_msm_device.argtypes = [i32, i32, u64p, ctypes.c_uint8, u64p, sz, u64p, u8p, vp]
     _lib = L
     return L
 

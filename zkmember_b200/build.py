@@ -23,6 +23,8 @@ UNITS = [   # the slowest units first: with fewer cores than units they must sta
     "zkm_msm_bw6.cu",
     "zkm_msm_g2_bls.cu",
     "zkm_msm_bw6_pair.cu",
+    "zkm_fixed_base_bw6.cu",
+    "zkm_fixed_base_bls.cu",
     "zkm_api.cu",
     "zkm_ntt_bls.cu",
     "zkm_ntt_bn.cu",
@@ -31,6 +33,7 @@ UNITS = [   # the slowest units first: with fewer cores than units they must sta
     "zkm_msm_g1_bn.cu",
     "zkm_msm_g2_bn.cu",
     "zkm_ntt_bw6.cu",
+    "zkm_fixed_base_bn.cu",
 ]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -58,6 +61,9 @@ UNIT_HEADERS = {
     "zkm_ntt_bw6.cu": ["zkm_ntt.cuh"],
     "zkm_msm_bw6.cu": ["zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
     "zkm_msm_bw6_pair.cu": ["zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
+    "zkm_fixed_base_bls.cu": ["zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
+    "zkm_fixed_base_bn.cu": ["zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
+    "zkm_fixed_base_bw6.cu": ["zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
 }
 
 

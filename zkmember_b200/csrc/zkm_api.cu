@@ -1409,6 +1409,51 @@ int32_t zkm_msm_window_bits(int32_t curve, int32_t group, size_t n) {
     return msm_auto_window_bits(curve, group, n);
 }
 
+int32_t zkm_fixed_base_msm(int32_t curve, int32_t group, const uint64_t* base_xy, uint8_t base_inf, const uint64_t* scalars,
+                           size_t n, uint64_t* out_xy, uint8_t* out_inf) {
+    return guarded([&] {
+        check_curve_group(curve, group);
+        if (n && (!base_xy || !scalars || !out_xy || !out_inf)) ZKM_FAIL(ZKM_ERR_ARG, "null pointer");
+        LaneGuard lane(pick_host_call_device());
+        Context* c = lane.c;
+        if (n == 0) return;
+        ZKM_CUDA(cudaSetDevice(c->device));
+        const size_t sbytes = (size_t)fr_words(curve) * 8, xyb = 2 * (size_t)coord_words(curve, group) * 8;
+        StreamScope scope(c, c->stream);
+        uint64_t* d_scal = (uint64_t*)c->io_scalars.get(n * sbytes);
+        uint64_t* d_xy = (uint64_t*)c->io_bases.get(n * xyb);
+        uint8_t* d_inf = (uint8_t*)c->io_inf.get(n);
+        uint32_t* d_flag = (uint32_t*)c->io_out.get(16);
+        ZKM_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(uint32_t), c->stream));
+        h2d(d_scal, scalars, n * sbytes, c->stream);
+        fixed_base_run(c, curve, group, base_xy, base_inf != 0, d_scal, n, d_xy, d_inf, d_flag, c->stream);
+        uint32_t* h_flag = (uint32_t*)c->pin_in.get(16);
+        ZKM_CUDA(cudaMemcpyAsync(out_xy, d_xy, n * xyb, cudaMemcpyDeviceToHost, c->stream));
+        ZKM_CUDA(cudaMemcpyAsync(out_inf, d_inf, n, cudaMemcpyDeviceToHost, c->stream));
+        ZKM_CUDA(cudaMemcpyAsync(h_flag, d_flag, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        ZKM_CUDA(cudaStreamSynchronize(c->stream));
+        if (*h_flag) ZKM_FAIL(ZKM_ERR_SCALAR_RANGE, "a scalar-field element is not below the modulus");
+    });
+}
+
+int32_t zkm_fixed_base_msm_device(int32_t curve, int32_t group, const uint64_t* base_xy, uint8_t base_inf, const uint64_t* d_scalars,
+                                  size_t n, uint64_t* d_out_xy, uint8_t* d_out_inf, void* stream) {
+    return guarded([&] {
+        check_curve_group(curve, group);
+        if (n && (!base_xy || !d_scalars || !d_out_xy || !d_out_inf)) ZKM_FAIL(ZKM_ERR_ARG, "null pointer");
+        if (((uintptr_t)d_scalars | (uintptr_t)d_out_xy) & 15) ZKM_FAIL(ZKM_ERR_ARG, "device pointers must be 16-byte aligned");
+        if (device_count_initialised() == 0) ZKM_FAIL(ZKM_ERR_NOT_INIT, "zkm_init() has not been called (or failed)");
+        const int home = n ? home_device_of(d_out_xy) : 0;
+        cudaStream_t s = call_stream(home, stream);
+        LaneGuard lane(home, s);
+        Context* c = lane.c;
+        if (n == 0) return;
+        ZKM_CUDA(cudaSetDevice(c->device));
+        StreamScope scope(c, s);
+        fixed_base_run(c, curve, group, base_xy, base_inf != 0, d_scalars, n, d_out_xy, d_out_inf, nullptr, s);
+    });
+}
+
 int32_t zkm_testgen_progression_device(int32_t curve, int32_t group, uint64_t a0, uint64_t d, size_t n,
                                        uint64_t* d_bases_xy, void* stream) {
     return guarded([&] {

@@ -324,6 +324,9 @@ void points_sum_run(Context* c, int curve, int group, const uint64_t* d_points, 
 void testgen_progression(Context* c, int curve, int group, uint64_t a0, uint64_t d, size_t n, uint64_t* d_out,
                          cudaStream_t stream);
 int msm_auto_window_bits(int curve, int group, size_t n);
+// out[i] = s_i * base (zkm_fixed_base.cuh); base_xy: host record; d_flag: null or a zeroed device word (bit 0: s_i >= r)
+void fixed_base_run(Context* c, int curve, int group, const uint64_t* base_xy, bool base_inf, const uint64_t* d_scalars, size_t n,
+                    uint64_t* d_out_xy, uint8_t* d_out_inf, uint32_t* d_flag, cudaStream_t stream);
 void note_profiled_lane(Context* c);   // zkm_profile_last_msm* report the lane that ran the last profiled MSM
 
 // 128-bit vectorised global access for field elements (N is a multiple of 4 limbs)

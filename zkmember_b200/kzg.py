@@ -3,6 +3,7 @@
     KZG10.commit(powers, coeffs[, gamma_powers, blinding_coeffs])   `KZG10::commit`  (src/kzg10/mod.rs)
     KZG10.commit_batch(powers, [coeffs, ...])                        the commitments of one prover round in one call
     KZG10.open(powers, coeffs, point[, gamma_powers, blinding])      `KZG10::open`: witness polynomial + its commitment
+    KZG10.setup(curve, max_degree, beta, g, gamma_g)                 `KZG10::setup`: the two power vectors of the SRS
 
 reached from /root/reference/benches/marlin.rs:202,311 through MarlinKZG10::{commit, open}.  Same meaning as upstream:
 `commit` skips the leading zero coefficients, converts with `into_repr()` and runs
@@ -20,7 +21,8 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _lib
-from .msm import AffinePoint, RegisteredBases, coord_words, _curve_id
+from .msm import AffinePoint, FixedBaseMSM, RegisteredBases, coord_words, _curve_id
+from .serialize import FR_MODULUS
 
 
 class Powers(RegisteredBases):
@@ -45,7 +47,48 @@ def _p(a):
     return ctypes.c_void_p(a.ctypes.data if a is not None and a.size else 0)
 
 
+@dataclass
+class UniversalParams:
+    """The group vectors of ark_poly_commit::kzg10::UniversalParams that KZG10::setup builds by fixed-base batches
+    (Montgomery affine records + infinity bytes)."""
+    powers_of_g: np.ndarray            # (max_degree + 1, 2 W): beta^i g
+    powers_of_g_inf: np.ndarray
+    powers_of_gamma_g: np.ndarray      # (max_degree + 2, 2 W): beta^i gamma_g, with the extra power upstream appends
+    powers_of_gamma_g_inf: np.ndarray
+
+
+def _powers_of_beta(curve: int, beta, count: int) -> np.ndarray:
+    """Montgomery limbs of beta^0 .. beta^(count - 1), computed on the host like upstream's `cur *= &beta` loop."""
+    S = _lib.FR_WORDS[curve]
+    r = FR_MODULUS[curve]
+    R = 1 << (64 * S)
+    b_mont = int.from_bytes(np.ascontiguousarray(beta, dtype=np.uint64).reshape(S).tobytes(), "little")
+    if b_mont >= r:
+        raise ValueError("beta is not a canonical Montgomery Fr element")
+    b = b_mont * pow(R, -1, r) % r
+    out = bytearray(8 * S * count)
+    cur = R % r                        # Montgomery one; mont(beta^i) = mont(beta^(i-1)) * beta mod r
+    for i in range(count):
+        out[8 * S * i:8 * S * (i + 1)] = cur.to_bytes(8 * S, "little")
+        cur = cur * b % r
+    return np.frombuffer(bytes(out), dtype=np.uint64).reshape(count, S)
+
+
 class KZG10:
+    @staticmethod
+    def setup(curve, max_degree: int, beta, g, gamma_g) -> UniversalParams:
+        """KZG10::setup (ark-poly-commit 0.3.0 src/kzg10/mod.rs) after its random draws: `beta` is one Montgomery Fr
+        element (S words), `g` / `gamma_g` the two G1 generators (AffinePoint or 2 W words).  powers_of_g[i] = beta^i g
+        for i <= max_degree; powers_of_gamma_g[i] = beta^i gamma_g for i <= max_degree + 1 (upstream pushes one more
+        power so that up to max_degree queries can be supported).  Both vectors are fixed-base batches on the GPU."""
+        cid = _curve_id(curve)
+        if max_degree < 1:
+            raise ValueError("max_degree must be at least 1 (upstream: DegreeIsZero)")
+        pw = _powers_of_beta(cid, beta, max_degree + 2)
+        g_xy, g_inf = FixedBaseMSM.multi_scalar_mul(g, pw[:max_degree + 1], curve=cid, group=1)
+        gg_xy, gg_inf = FixedBaseMSM.multi_scalar_mul(gamma_g, pw, curve=cid, group=1)
+        return UniversalParams(g_xy, g_inf, gg_xy, gg_inf)
+
     @staticmethod
     def commit(powers: RegisteredBases, coeffs, gamma_powers: RegisteredBases | None = None, blinding_coeffs=None) -> AffinePoint:
         """coeffs: (d + 1, S) uint64 Montgomery Fr, low degree first (DensePolynomial::coeffs)."""

@@ -1,6 +1,7 @@
-"""Host-side mirror of ark-ec 0.3.0's variable-base MSM interface.
+"""Host-side mirror of ark-ec 0.3.0's MSM interfaces.
 
     VariableBaseMSM.multi_scalar_mul(bases, scalars) -> affine point
+    FixedBaseMSM.multi_scalar_mul(base, scalars)     -> n affine points s_i * base (the setup paths)
 
 replaces `ark_ec::msm::VariableBaseMSM::multi_scalar_mul` (src/msm/variable_base.rs; pin
 /root/reference/Cargo.lock:179-180) + `into_affine()`, the call ark-groth16's create_proof makes
@@ -141,6 +142,53 @@ class VariableBaseMSM:
         fn = L.zkm_msm_g1 if group == 1 else L.zkm_msm_g2
         _lib.check(fn(cid, _ptr(b), _ptr(inf), _ptr(s), n, _ptr(out), _ptr(oinf)))
         return AffinePoint(cid, group, out, bool(oinf[0]))
+
+
+def _base_record(base, cid: int, group: int):
+    """(xy words, infinity flag) of ONE affine base: an AffinePoint or its 2 W words."""
+    W = coord_words(cid, group)
+    if isinstance(base, AffinePoint):
+        if base.curve != cid or base.group != group:
+            raise ValueError("base is a point of curve %d group %d, not curve %d group %d" % (base.curve, base.group, cid, group))
+        xy, inf = base.xy, base.infinity
+    else:
+        xy, inf = base, False
+    xy = np.ascontiguousarray(xy, dtype=np.uint64)
+    if xy.size != 2 * W:
+        raise ValueError("base: expected %d words (one affine point), got %d" % (2 * W, xy.size))
+    return xy.reshape(2 * W), 1 if inf else 0
+
+
+class FixedBaseMSM:
+    """Namesake of ark_ec::msm::FixedBaseMSM: get_window_table + multi_scalar_mul + batch_normalization_into_affine in
+    one call (the window width is the library's choice)."""
+
+    @staticmethod
+    def multi_scalar_mul(base, scalars, curve="bls12_381", group: int = 1):
+        """s_i * base for every Montgomery Fr element s_i of `scalars` ((n, S) uint64, as upstream's &[G::ScalarField]).
+        Returns (xy (n, 2W) uint64 Montgomery affine, inf (n,) uint8).  An element >= r raises ZKM_ERR_SCALAR_RANGE."""
+        cid = _curve_id(curve)
+        if group not in (1, 2):
+            raise ValueError("group must be 1 or 2, got %r" % (group,))
+        W = coord_words(cid, group)
+        xy_b, inf_b = _base_record(base, cid, group)
+        s = _as_u64(scalars, FR_WORDS[cid], "scalars")
+        n = len(s)
+        out = np.zeros((n, 2 * W), dtype=np.uint64)
+        oinf = np.zeros(n, dtype=np.uint8)
+        _lib.check(_lib.lib().zkm_fixed_base_msm(cid, group, _ptr(xy_b), inf_b, _ptr(s), n, _ptr(out), _ptr(oinf)))
+        return out, oinf
+
+    @staticmethod
+    def multi_scalar_mul_device(base, d_scalars_ptr: int, n: int, d_out_xy_ptr: int, d_out_inf_ptr: int, curve="bls12_381",
+                                group: int = 1, stream: int = 0):
+        """Device-resident variant: n Montgomery scalars and the n affine records + infinity bytes stay in HBM; enqueued on
+        `stream` without a host wait.  Scalars are not range-checked here."""
+        cid = _curve_id(curve)
+        xy_b, inf_b = _base_record(base, cid, group)
+        _lib.check(_lib.lib().zkm_fixed_base_msm_device(cid, group, _ptr(xy_b), inf_b, ctypes.c_void_p(d_scalars_ptr), n,
+                                                        ctypes.c_void_p(d_out_xy_ptr), ctypes.c_void_p(d_out_inf_ptr),
+                                                        ctypes.c_void_p(stream)))
 
 
 def msm_window_bits(curve, group: int, n: int) -> int:
