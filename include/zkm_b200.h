@@ -172,6 +172,42 @@ int32_t zkm_fixed_base_msm_device(int32_t curve, int32_t group, const uint64_t* 
                                   const uint64_t* d_scalars, size_t n, uint64_t* d_out_xy, uint8_t* d_out_inf,
                                   void* stream);
 
+/* ---- Groth16 prover -------------------------------------------------------------------------------
+ * Replaces ark-groth16 0.3.0 create_proof_with_reduction_and_matrices (src/prover.rs) after synthesis: the witness
+ * map's FFTs, the five MSMs and the final assembly of Proof { a, b, c } in one call.
+ *
+ * zkm_groth16_pk_create: ark_groth16::ProvingKey on the device.  handles[5] are registrations (any flags) of h_query,
+ * l_query, a_query[1..], b_g1_query[1..], b_g2_query[1..] -- groups 1, 1, 1, 1, 2 of one curve, the last three of equal
+ * length.  The key holds references to them: the caller may release the handles afterwards.  g1_xy: 5 affine records
+ * (2 W1 words each) alpha_g1, beta_g1, delta_g1, a_query[0], b_g1_query[0] with g1_inf[5]; g2_xy: 3 records (2 W2
+ * words) beta_g2, delta_g2, b_g2_query[0] with g2_inf[3].  Builds a window table of delta_g1 and delta_g2 on every
+ * initialised device, so that the delta multiples of a proof need no doublings.  Unknown curve, wrong group or curve
+ * of a handle, or unequal query lengths give ZKM_ERR_ARG; an unknown handle ZKM_ERR_HANDLE. */
+int32_t zkm_groth16_pk_create(int32_t curve, const uint64_t* handles, const uint64_t* g1_xy, const uint8_t* g1_inf,
+                              const uint64_t* g2_xy, const uint8_t* g2_inf, uint64_t* pk_out);
+/* Releases the key (a call still using it keeps it alive until it returns); an unknown key gives ZKM_ERR_HANDLE. */
+int32_t zkm_groth16_pk_release(uint64_t pk);
+/* a, b, c: the 2^log_n evaluation vectors handed to R1CStoQAP::witness_map (Montgomery Fr, as zkm_witness_map).
+ * assignment = input_assignment[1..] || aux_assignment, canonical (into_repr), num_inputs + num_aux elements.
+ * r, s: canonical Fr (S64 words); 0 is legal.  All HOST pointers.  Writes Proof { a: G1, b: G2, c: G1 } as normalised
+ * affine records (zero = x 0, y 1, infinity byte 1).  Requires len(a_query) - 1 = num_inputs + num_aux,
+ * len(l_query) = num_aux and len(h_query) <= 2^log_n, else ZKM_ERR_ARG; a released key gives ZKM_ERR_HANDLE; an
+ * assignment element, r or s >= the scalar modulus gives ZKM_ERR_SCALAR_RANGE.  One pinned upload, the device form,
+ * one read-back. */
+int32_t zkm_groth16_prove(uint64_t pk, const uint64_t* a, const uint64_t* b, const uint64_t* c, uint32_t log_n,
+                          const uint64_t* assignment, size_t num_inputs, size_t num_aux, const uint64_t* r, const uint64_t* s,
+                          uint64_t* out_a_xy, uint8_t* out_a_inf, uint64_t* out_b_xy, uint8_t* out_b_inf,
+                          uint64_t* out_c_xy, uint8_t* out_c_inf);
+/* Device form: d_a, d_b, d_c (consumed: overwritten) and d_assignment are DEVICE pointers; d_out receives three packed
+ * records A (2 W1 + 1 words), B (2 W2 + 1), C (2 W1 + 1) whose last word is the flag of zkm_msm_registered_device:
+ * 0 finite, 1 infinity, 2 invalid (an assignment element, r or s >= the scalar modulus; all three records then carry
+ * 2).  r and s stay HOST pointers (passed to the kernels by value).  A fixed launch sequence on `stream`: witness map,
+ * into_repr of h, the five MSMs (concurrently, the b_g2 one on the device of its registration), the assembly; no
+ * device read-back, no host wait.  Concurrent calls from several host threads overlap on the GPU. */
+int32_t zkm_groth16_prove_device(uint64_t pk, uint64_t* d_a, uint64_t* d_b, uint64_t* d_c, uint32_t log_n,
+                                 const uint64_t* d_assignment, size_t num_inputs, size_t num_aux, const uint64_t* r,
+                                 const uint64_t* s, uint64_t* d_out, void* stream);
+
 /* ---- radix-2 NTT ------------------------------------------------------------------------------
  * Replaces ark_poly::Radix2EvaluationDomain::{fft_in_place, ifft_in_place, coset_fft_in_place,
  * coset_ifft_in_place} (ark-poly 0.3.0 src/domain/radix2/{mod,fft}.rs, src/domain/mod.rs) on the

@@ -11,6 +11,7 @@
 //   zkm::witness_map(domain, a, b, c)                           ark-groth16 0.3.0 src/r1cs_to_qap.rs
 //   zkm::ProvingKeyBases / KZG10::commit                        registered bases (pk / SRS reuse)
 //   zkm::serialize(point) / zkm::Proof<Curve>::serialize()      arkworks' compressed CanonicalSerialize (host code)
+//   zkm::Groth16ProvingKey<Curve> / zkm::create_proof            ark-groth16 0.3.0 src/prover.rs (after synthesis)
 //
 // Types are plain structs with arkworks' memory layout: Fp256 = 4 x u64 Montgomery limbs, Fp384 = 6,
 // BigInteger256 = 4 x u64 canonical limbs (BigInteger384 = 6 for BW6-761), GroupAffine{x, y, infinity}.  Errors of the C ABI become
@@ -453,5 +454,68 @@ struct Proof {
         return out;
     }
 };
+
+// ark_groth16::ProvingKey on the device (zkm_groth16_pk_create).  a_query, b_g1_query, b_g2_query are the FULL vectors:
+// entry 0 (the constant-one variable) goes to the key as a point, entries 1.. are registered; the key keeps the
+// registrations alive, the RAII members below only drop this object's own references.
+template <class Curve>
+class Groth16ProvingKey {
+public:
+    Groth16ProvingKey(const G1Affine<Curve>& alpha_g1, const G1Affine<Curve>& beta_g1, const G2Affine<Curve>& beta_g2,
+                      const G1Affine<Curve>& delta_g1, const G2Affine<Curve>& delta_g2, const std::vector<G1Affine<Curve>>& a_query,
+                      const std::vector<G1Affine<Curve>>& b_g1_query, const std::vector<G2Affine<Curve>>& b_g2_query,
+                      const std::vector<G1Affine<Curve>>& h_query, const std::vector<G1Affine<Curve>>& l_query, bool precompute = true)
+        : h_(h_query, precompute), l_(l_query, precompute), a_(tail(a_query), precompute), b1_(tail(b_g1_query), precompute),
+          b2_(tail(b_g2_query), precompute) {
+        const uint64_t handles[5] = {h_.handle(), l_.handle(), a_.handle(), b1_.handle(), b2_.handle()};
+        std::vector<uint64_t> g1, g2;
+        std::vector<uint8_t> g1_inf, g2_inf;
+        detail::pack<Curve, 1>({alpha_g1, beta_g1, delta_g1, first(a_query), first(b_g1_query)}, 5, g1, g1_inf);
+        detail::pack<Curve, 2>({beta_g2, delta_g2, first(b_g2_query)}, 3, g2, g2_inf);
+        check(zkm_groth16_pk_create(Curve::ID, handles, g1.data(), g1_inf.data(), g2.data(), g2_inf.data(), &handle_),
+              "zkm_groth16_pk_create");
+    }
+    ~Groth16ProvingKey() { if (handle_) zkm_groth16_pk_release(handle_); }
+    Groth16ProvingKey(const Groth16ProvingKey&) = delete;
+    Groth16ProvingKey& operator=(const Groth16ProvingKey&) = delete;
+    uint64_t handle() const { return handle_; }
+
+private:
+    template <class T>
+    static std::vector<T> tail(const std::vector<T>& v) { return v.empty() ? v : std::vector<T>(v.begin() + 1, v.end()); }
+    template <class T>
+    static T first(const std::vector<T>& v) {
+        if (v.empty()) throw Error(ZKM_ERR_ARG, "Groth16ProvingKey: empty query vector");
+        return v[0];
+    }
+    RegisteredBases<Curve, 1> h_, l_, a_, b1_;
+    RegisteredBases<Curve, 2> b2_;
+    uint64_t handle_ = 0;
+};
+
+// create_proof_with_reduction_and_matrices after synthesis: a, b, c are the evaluation vectors of the witness map
+// (Montgomery Fr, 2^k elements), inputs = input_assignment[1..] and aux the canonical assignments, r and s canonical.
+template <class Curve>
+Proof<Curve> create_proof(const Groth16ProvingKey<Curve>& pk, const typename Curve::BigInt& r, const typename Curve::BigInt& s,
+                          const std::vector<typename Curve::Fr>& a, const std::vector<typename Curve::Fr>& b,
+                          const std::vector<typename Curve::Fr>& c, const std::vector<typename Curve::BigInt>& inputs,
+                          const std::vector<typename Curve::BigInt>& aux) {
+    uint32_t log_n = 0;
+    while (((size_t)1 << log_n) < a.size()) log_n++;
+    if (a.empty() || ((size_t)1 << log_n) != a.size() || b.size() != a.size() || c.size() != a.size())
+        throw Error(ZKM_ERR_ARG, "create_proof: a, b, c must have the same power-of-two length");
+    std::vector<typename Curve::BigInt> z(inputs);
+    z.insert(z.end(), aux.begin(), aux.end());
+    typedef typename G1Affine<Curve>::Coord C1;
+    typedef typename G2Affine<Curve>::Coord C2;
+    std::vector<uint64_t> oa(2 * sizeof(C1) / 8), ob(2 * sizeof(C2) / 8), oc(2 * sizeof(C1) / 8);
+    uint8_t ia = 0, ib = 0, ic = 0;
+    check(zkm_groth16_prove(pk.handle(), reinterpret_cast<const uint64_t*>(a.data()), reinterpret_cast<const uint64_t*>(b.data()),
+                            reinterpret_cast<const uint64_t*>(c.data()), log_n, reinterpret_cast<const uint64_t*>(z.data()),
+                            inputs.size(), aux.size(), reinterpret_cast<const uint64_t*>(&r), reinterpret_cast<const uint64_t*>(&s),
+                            oa.data(), &ia, ob.data(), &ib, oc.data(), &ic),
+          "zkm_groth16_prove");
+    return Proof<Curve>{detail::unpack<Curve, 1>(oa, ia), detail::unpack<Curve, 2>(ob, ib), detail::unpack<Curve, 1>(oc, ic)};
+}
 
 }  // namespace zkm

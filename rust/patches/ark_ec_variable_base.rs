@@ -52,9 +52,11 @@ impl VariableBaseMSM {
 }
 
 /// (curve id, group, u64 words per coordinate, u64 words per scalar) of include/zkm_b200.h.
-/// Crate-visible: the fixed-base patch (ark_ec_fixed_base.rs) routes with the same table.
+/// Public (hidden): the fixed-base patch (ark_ec_fixed_base.rs) and the ark-groth16 prover fork
+/// (ark_groth16_prover.rs) route with the same table.
 #[derive(Clone, Copy)]
-pub(crate) struct GroupId { pub(crate) curve: i32, pub(crate) group: i32, pub(crate) coord_words: usize, pub(crate) scalar_words: usize }
+#[doc(hidden)]
+pub struct GroupId { pub curve: i32, pub group: i32, pub coord_words: usize, pub scalar_words: usize }
 
 // Moduli of the base PRIME fields the library implements (little-endian u64 limbs; the published curve parameters,
 // the same numbers as oracle/py/params.py).  Routing compares the type's own `FpParameters::MODULUS` with these, so it
@@ -69,7 +71,8 @@ const BW6_761_FQ: [u64; 12] = [
 ];
 const BW6_761_FR: [u64; 6] = [0x8508c00000000001, 0x170b5d4430000000, 0x1ef3622fba094800, 0x1a22d9f300f5138f, 0xc63b05c06ca1493b, 0x01ae3a4617c510ea];
 
-pub(crate) fn gpu_group<G: AffineCurve>() -> Option<GroupId> {
+#[doc(hidden)]
+pub fn gpu_group<G: AffineCurve>() -> Option<GroupId> {
     type BasePrime<G> = <<G as AffineCurve>::BaseField as Field>::BasePrimeField;
     let q = <<BasePrime<G> as PrimeField>::Params as FpParameters>::MODULUS;
     let r = <<G::ScalarField as PrimeField>::Params as FpParameters>::MODULUS;
@@ -108,7 +111,8 @@ fn fingerprint<G: AffineCurve>(bases: &[G], words: usize) -> u64 {
     h
 }
 
-fn registered<G: AffineCurve>(id: GroupId, bases: &[G]) -> u64 {
+#[doc(hidden)]
+pub fn registered<G: AffineCurve>(id: GroupId, bases: &[G]) -> u64 {
     let key = (bases.as_ptr() as usize, bases.len(), id.curve, id.group);
     let fp = fingerprint(bases, id.coord_words);
     let mut cache = CACHE.lock().unwrap();

@@ -49,6 +49,16 @@ extern "C" {
                           stream: *mut c_void) -> i32;
     pub fn zkm_msm_registered_device(handle: u64, offset: usize, d_scalars: *const u64, n: usize, d_out: *mut u64,
                                      stream: *mut c_void) -> i32;
+    pub fn zkm_groth16_pk_create(curve: i32, handles: *const u64, g1_xy: *const u64, g1_inf: *const u8, g2_xy: *const u64,
+                                 g2_inf: *const u8, pk_out: *mut u64) -> i32;
+    pub fn zkm_groth16_pk_release(pk: u64) -> i32;
+    pub fn zkm_groth16_prove(pk: u64, a: *const u64, b: *const u64, c: *const u64, log_n: u32, assignment: *const u64,
+                             num_inputs: usize, num_aux: usize, r: *const u64, s: *const u64, out_a_xy: *mut u64,
+                             out_a_inf: *mut u8, out_b_xy: *mut u64, out_b_inf: *mut u8, out_c_xy: *mut u64,
+                             out_c_inf: *mut u8) -> i32;
+    pub fn zkm_groth16_prove_device(pk: u64, d_a: *mut u64, d_b: *mut u64, d_c: *mut u64, log_n: u32,
+                                    d_assignment: *const u64, num_inputs: usize, num_aux: usize, r: *const u64,
+                                    s: *const u64, d_out: *mut u64, stream: *mut c_void) -> i32;
 }
 
 /// Panics with the library's message: the upstream functions are infallible and there is deliberately

@@ -34,6 +34,7 @@ SYMBOLS = [
     "zkm_init_mask", "zkm_init_devices", "zkm_initialised_devices", "zkm_bases_register_ex", "zkm_kzg_commit_batch",
     "zkm_kzg_commit_hiding", "zkm_kzg_open", "zkm_profile_last_msm_counts", "zkm_msm_cache_clear", "zkm_msm_cache_stats",
     "zkm_fixed_base_msm", "zkm_fixed_base_msm_device",
+    "zkm_groth16_pk_create", "zkm_groth16_pk_release", "zkm_groth16_prove", "zkm_groth16_prove_device",
 ]
 
 # zkm_bases_register_ex flags (include/zkm_b200.h)
@@ -109,6 +110,10 @@ def load():
     L.zkm_testgen_progression_device.argtypes = [i32, i32, u64, u64, sz, u64p, vp]
     L.zkm_fixed_base_msm.argtypes = [i32, i32, u64p, ctypes.c_uint8, u64p, sz, u64p, u8p]
     L.zkm_fixed_base_msm_device.argtypes = [i32, i32, u64p, ctypes.c_uint8, u64p, sz, u64p, u8p, vp]
+    L.zkm_groth16_pk_create.argtypes = [i32, ctypes.c_void_p, u64p, u8p, u64p, u8p, ctypes.POINTER(u64)]
+    L.zkm_groth16_pk_release.argtypes = [u64]
+    L.zkm_groth16_prove.argtypes = [u64, u64p, u64p, u64p, u32, u64p, sz, sz, u64p, u64p, u64p, u8p, u64p, u8p, u64p, u8p]
+    L.zkm_groth16_prove_device.argtypes = [u64, u64p, u64p, u64p, u32, u64p, sz, sz, u64p, u64p, u64p, vp]
     _lib = L
     return L
 

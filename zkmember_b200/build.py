@@ -34,6 +34,9 @@ UNITS = [   # the slowest units first: with fewer cores than units they must sta
     "zkm_msm_g2_bn.cu",
     "zkm_ntt_bw6.cu",
     "zkm_fixed_base_bn.cu",
+    "zkm_groth16_bw6.cu",
+    "zkm_groth16_bls.cu",
+    "zkm_groth16_bn.cu",
 ]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -50,7 +53,7 @@ def _nvcc() -> str:
 
 BASE_HEADERS = ["zkm_common.cuh", "zkm_curve.cuh", "zkm_field.cuh", "zkm_fpmul_u.cuh", "zkm_arith.cuh", "zkm_constants.cuh"]
 UNIT_HEADERS = {
-    "zkm_api.cu": [],
+    "zkm_api.cu": ["zkm_groth16_ops.cuh"],
     "zkm_ntt_bls.cu": ["zkm_ntt.cuh"],
     "zkm_ntt_bn.cu": ["zkm_ntt.cuh"],
     "zkm_msm.cu": ["zkm_msm.cuh"],
@@ -64,6 +67,12 @@ UNIT_HEADERS = {
     "zkm_fixed_base_bls.cu": ["zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
     "zkm_fixed_base_bn.cu": ["zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
     "zkm_fixed_base_bw6.cu": ["zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh", "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
+    "zkm_groth16_bls.cu": ["zkm_groth16.cuh", "zkm_groth16_ops.cuh", "zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh",
+                           "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
+    "zkm_groth16_bn.cu": ["zkm_groth16.cuh", "zkm_groth16_ops.cuh", "zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh",
+                          "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
+    "zkm_groth16_bw6.cu": ["zkm_groth16.cuh", "zkm_groth16_ops.cuh", "zkm_fixed_base.cuh", "zkm_msm.cuh", "zkm_msm_curve.cuh",
+                           "zkm_msm_affine.cuh", "zkm_msm_quad.cuh"],
 }
 
 

@@ -8,11 +8,44 @@
 #include <thread>
 
 #include "zkm_common.cuh"
+#include "zkm_groth16_ops.cuh"
 
 namespace zkm {
 
 static thread_local char t_err[512] = "";
 std::atomic<uint64_t> g_launches{0};
+
+// A Groth16 proving key (zkm_groth16_pk_create): references to the five query registrations, the key's eight points
+// as records and the window tables of delta_g1 / delta_g2, on every initialised device (a proof runs where its
+// output lives).
+struct G16Key {
+    int curve = 0;
+    size_t m = 0;                                 // num_inputs + num_aux = len(a_query) - 1
+    std::shared_ptr<BasesReg> reg[5];             // h, l, a[1..], b_g1[1..], b_g2[1..]
+    bool delta1_inf = false, delta2_inf = false;
+    struct Dev {
+        int ordinal = -1;
+        uint64_t* d_key = nullptr;                // 5 G1 records, then 3 G2 records
+        char* d_tab1 = nullptr;
+        char* d_tab2 = nullptr;
+    };
+    std::vector<Dev> dev;                         // by device index
+    ~G16Key() {
+        int cur = -1;
+        cudaGetDevice(&cur);
+        for (Dev& d : dev) {
+            if (d.ordinal < 0 || cudaSetDevice(d.ordinal) != cudaSuccess) { cudaGetLastError(); continue; }
+            // no proof may still be reading the key: the same drain as ~BasesReg (cudaFree would synchronise anyway)
+            cudaDeviceSynchronize();
+            if (d.d_key) cudaFree(d.d_key);
+            if (d.d_tab1) cudaFree(d.d_tab1);
+            if (d.d_tab2) cudaFree(d.d_tab2);
+            cudaGetLastError();
+        }
+        if (cur >= 0) cudaSetDevice(cur);
+        cudaGetLastError();
+    }
+};
 
 // Process-wide state: the initialised devices (index 0 = primary), their lanes, options, registrations.
 struct Global {
@@ -22,6 +55,7 @@ struct Global {
     Options opt;
     std::mutex reg_mu;                            // guards `bases` / `next_handle`
     std::map<uint64_t, std::shared_ptr<BasesReg>> bases;
+    std::map<uint64_t, std::shared_ptr<G16Key>> pks;   // Groth16 proving keys (same handle counter)
     uint64_t next_handle = 1;
     // registration cache of the literal multi_scalar_mul(bases, scalars) call (zkm_msm_g1 / zkm_msm_g2)
     struct CacheKey {
@@ -483,37 +517,61 @@ struct DevItem {
     size_t offset, n;
     const uint64_t* d_scalars;
     uint64_t* d_out;
+    // non-null: when the item runs as one job on a lane of its own, its completion event is handed back here instead
+    // of being joined into the caller's stream (the caller waits for it and destroys it); null on return otherwise
+    cudaEvent_t* done = nullptr;
 };
-static void msm_items_device(std::vector<DevItem>& items, int home, cudaStream_t caller_or_null) {
+struct ItemsPlan {
     struct Flat { size_t item, k; Job job; };
     std::vector<Flat> flat;
-    std::vector<size_t> njobs(items.size()), goff(items.size(), 0);
+    std::vector<size_t> njobs, goff;
     size_t gbytes = 0;       // sharded items gather their partial records at goff[item] + k * rec_bytes (copies only)
+    bool fast = false;
+    std::vector<int> devs;           // lane 0: the home lane; lanes 1..: one per job
+    std::vector<uint64_t> keys;      // lane affinity: the part of the registration a job runs over (same workspace sizes)
+};
+static ItemsPlan plan_items(const std::vector<DevItem>& items, int home) {
+    ItemsPlan p;
+    p.njobs.assign(items.size(), 0);
+    p.goff.assign(items.size(), 0);
     for (size_t i = 0; i < items.size(); i++) {
         std::vector<Job> jobs = split_jobs(*items[i].reg, items[i].offset, items[i].n);
-        njobs[i] = jobs.size();
-        for (size_t k = 0; k < jobs.size(); k++) flat.push_back(Flat{i, k, jobs[k]});
+        p.njobs[i] = jobs.size();
+        for (size_t k = 0; k < jobs.size(); k++) p.flat.push_back(ItemsPlan::Flat{i, k, jobs[k]});
         if (jobs.size() > 1) {
-            goff[i] = gbytes;
-            gbytes += (jobs.size() * rec_bytes(items[i].reg->curve, items[i].reg->group) + 15) & ~(size_t)15;
+            p.goff[i] = p.gbytes;
+            p.gbytes += (jobs.size() * rec_bytes(items[i].reg->curve, items[i].reg->group) + 15) & ~(size_t)15;
         }
     }
-    const bool fast = items.size() == 1 && flat.size() == 1 && flat[0].job.part->dev == home;
-    // lane 0: the home lane; lanes 1..: one per job -- all taken together (no hold-and-wait between concurrent calls)
-    std::vector<int> devs{home};
-    std::vector<uint64_t> keys{0};     // lane affinity: the part of the registration a job runs over (same workspace sizes)
-    if (!fast)
-        for (const Flat& f : flat) {
-            devs.push_back(f.job.part->dev);
-            keys.push_back(lane_key(f.job.part, f.job.count));
+    p.fast = items.size() == 1 && p.flat.size() == 1 && p.flat[0].job.part->dev == home;
+    p.devs = {home};
+    p.keys = {0};
+    if (!p.fast)
+        for (const ItemsPlan::Flat& f : p.flat) {
+            p.devs.push_back(f.job.part->dev);
+            p.keys.push_back(lane_key(f.job.part, f.job.count));
         }
-    MultiLaneGuard lanes(devs, caller_or_null, &keys);
-    Context* hc = lanes.c[0];
+    return p;
+}
+static void run_items(std::vector<DevItem>& items, const ItemsPlan& plan, Context* const* lanes, cudaStream_t caller);
+static void msm_items_device(std::vector<DevItem>& items, int home, cudaStream_t caller_or_null) {
+    const ItemsPlan plan = plan_items(items, home);
+    // all lanes taken together (no hold-and-wait between concurrent calls)
+    MultiLaneGuard lanes(plan.devs, caller_or_null, &plan.keys);
+    run_items(items, plan, lanes.c.data(), caller_or_null);
+}
+// the MSMs of `items` on the lanes of plan.devs (lanes[0]: the home lane)
+static void run_items(std::vector<DevItem>& items, const ItemsPlan& plan, Context* const* lanes, cudaStream_t caller) {
+    const std::vector<ItemsPlan::Flat>& flat = plan.flat;
+    const std::vector<size_t>& njobs = plan.njobs;
+    const std::vector<size_t>& goff = plan.goff;
+    for (DevItem& it : items)
+        if (it.done) *it.done = nullptr;
+    Context* hc = lanes[0];
     ZKM_CUDA(cudaSetDevice(hc->device));
-    cudaStream_t caller = caller_or_null;
     StreamScope hscope(hc, caller);
     // fast path: one job on the caller's device -> no threads, no events, the caller's stream itself
-    if (fast) {
+    if (plan.fast) {
         const BasesReg& r = *items[0].reg;
         const size_t sbytes = (size_t)fr_words(r.curve) * 8;
         run_part(hc, r, flat[0].job, (const uint64_t*)((const char*)items[0].d_scalars + flat[0].job.scal_off * sbytes),
@@ -526,7 +584,7 @@ static void msm_items_device(std::vector<DevItem>& items, int home, cudaStream_t
             msm_run(hc, r.curve, r.group, nullptr, nullptr, nullptr, 0, items[i].d_out, caller);   // identity
         }
     if (flat.empty()) return;
-    char* d_gather = (char*)hc->gather.get(gbytes + 16);
+    char* d_gather = (char*)hc->gather.get(plan.gbytes + 16);
     cudaEvent_t ev_in;
     ZKM_CUDA(cudaEventCreateWithFlags(&ev_in, cudaEventDisableTiming));
     ZKM_CUDA(cudaEventRecord(ev_in, caller));
@@ -538,11 +596,11 @@ static void msm_items_device(std::vector<DevItem>& items, int home, cudaStream_t
     for (size_t f = 0; f < flat.size(); f++) {
         th.emplace_back([&, f] {
             rc[f] = guarded([&] {
-                const Flat& fj = flat[f];
+                const ItemsPlan::Flat& fj = flat[f];
                 const DevItem& it = items[fj.item];
                 const BasesReg& r = *it.reg;
                 const size_t sbytes = (size_t)fr_words(r.curve) * 8, rb = rec_bytes(r.curve, r.group);
-                Context* c = lanes.c[1 + f];
+                Context* c = lanes[1 + f];
                 ZKM_CUDA(cudaSetDevice(c->device));
                 cudaStream_t s = c->stream;
                 StreamScope scope(c, s);
@@ -575,7 +633,10 @@ static void msm_items_device(std::vector<DevItem>& items, int home, cudaStream_t
     ZKM_CUDA(cudaSetDevice(hc->device));
     int32_t first = ZKM_OK;
     for (size_t f = 0; f < flat.size(); f++) {
-        if (ev_out[f]) {
+        DevItem& it = items[flat[f].item];
+        if (ev_out[f] && it.done && njobs[flat[f].item] == 1 && rc[f] == ZKM_OK) {
+            *it.done = ev_out[f];      // joined by the caller
+        } else if (ev_out[f]) {
             cudaStreamWaitEvent(caller, ev_out[f], 0);
             cudaEventDestroy(ev_out[f]);
         }
@@ -585,7 +646,15 @@ static void msm_items_device(std::vector<DevItem>& items, int home, cudaStream_t
         }
     }
     cudaEventDestroy(ev_in);
-    if (first != ZKM_OK) throw ZkmError{first};
+    if (first != ZKM_OK) {
+        for (DevItem& it : items)
+            if (it.done && *it.done) {
+                cudaStreamWaitEvent(caller, *it.done, 0);
+                cudaEventDestroy(*it.done);
+                *it.done = nullptr;
+            }
+        throw ZkmError{first};
+    }
     for (size_t i = 0; i < items.size(); i++)
         if (njobs[i] > 1) {
             const BasesReg& r = *items[i].reg;
@@ -852,6 +921,195 @@ static int32_t init_devices(const int32_t* devices, int32_t count) {
     });
 }
 
+// ------------------------------------------------------------------------------------------ Groth16 prover
+static std::shared_ptr<G16Key> g16_lookup(uint64_t pk) {
+    if (!g) ZKM_FAIL(ZKM_ERR_NOT_INIT, "zkm_init() has not been called (or failed)");
+    std::lock_guard<std::mutex> rl(g->reg_mu);
+    auto it = g->pks.find(pk);
+    if (it == g->pks.end()) ZKM_FAIL(ZKM_ERR_HANDLE, "unknown Groth16 proving key %llu", (unsigned long long)pk);
+    return it->second;
+}
+
+static uint64_t g16_create(int curve, const uint64_t* handles, const uint64_t* g1_xy, const uint8_t* g1_inf, const uint64_t* g2_xy,
+                           const uint8_t* g2_inf) {
+    if (!curve_known(curve)) ZKM_FAIL(ZKM_ERR_ARG, "unknown curve id %d", curve);
+    if (!handles || !g1_xy || !g1_inf || !g2_xy || !g2_inf) ZKM_FAIL(ZKM_ERR_ARG, "null pointer");
+    auto key = std::make_shared<G16Key>();
+    key->curve = curve;
+    static const char* names[5] = {"h_query", "l_query", "a_query", "b_g1_query", "b_g2_query"};
+    for (int i = 0; i < 5; i++) {
+        key->reg[i] = lookup(handles[i], 0, 0);
+        const int want = i == G16_B2 ? 2 : 1;
+        if (key->reg[i]->curve != curve || key->reg[i]->group != want)
+            ZKM_FAIL(ZKM_ERR_ARG, "%s: registration of curve %d group %d, expected curve %d group %d", names[i], key->reg[i]->curve,
+                     key->reg[i]->group, curve, want);
+    }
+    key->m = key->reg[G16_A]->n;
+    if (key->reg[G16_B1]->n != key->m || key->reg[G16_B2]->n != key->m)
+        ZKM_FAIL(ZKM_ERR_ARG, "a_query, b_g1_query and b_g2_query differ in length (%zu, %zu, %zu after entry 0)", key->m,
+                 key->reg[G16_B1]->n, key->reg[G16_B2]->n);
+    const size_t xy1 = 2 * (size_t)coord_words(curve, 1), xy2 = 2 * (size_t)coord_words(curve, 2);
+    const size_t rw1 = xy1 + 1, rw2 = xy2 + 1;
+    std::vector<uint64_t> rec(5 * rw1 + 3 * rw2, 0);
+    for (int i = 0; i < 5; i++) {
+        memcpy(&rec[i * rw1], g1_xy + i * xy1, xy1 * 8);
+        rec[i * rw1 + xy1] = g1_inf[i] ? 1 : 0;
+    }
+    for (int j = 0; j < 3; j++) {
+        memcpy(&rec[5 * rw1 + j * rw2], g2_xy + j * xy2, xy2 * 8);
+        rec[5 * rw1 + j * rw2 + xy2] = g2_inf[j] ? 1 : 0;
+    }
+    key->delta1_inf = g1_inf[G16_DELTA] != 0;
+    key->delta2_inf = g2_inf[G16_DELTA2] != 0;
+    const G16Ops ops = groth16_ops(curve);
+    const int ndev = device_count_initialised();
+    if (ndev == 0) ZKM_FAIL(ZKM_ERR_NOT_INIT, "zkm_init() has not been called (or failed)");
+    key->dev.resize(ndev);
+    for (int d = 0; d < ndev; d++) {
+        LaneGuard lane(d);
+        Context* c = lane.c;
+        ZKM_CUDA(cudaSetDevice(c->device));
+        G16Key::Dev& kd = key->dev[d];
+        kd.ordinal = c->device;
+        StreamScope scope(c, c->stream);
+        ZKM_CUDA(malloc_retry((void**)&kd.d_key, rec.size() * 8));
+        h2d(kd.d_key, rec.data(), rec.size() * 8, c->stream);
+        if (!key->delta1_inf) {
+            ZKM_CUDA(malloc_retry((void**)&kd.d_tab1, ops.table_bytes(1)));
+            ops.table(c, 1, g1_xy + G16_DELTA * xy1, kd.d_tab1, c->stream);
+        }
+        if (!key->delta2_inf) {
+            ZKM_CUDA(malloc_retry((void**)&kd.d_tab2, ops.table_bytes(2)));
+            ops.table(c, 2, g2_xy + G16_DELTA2 * xy2, kd.d_tab2, c->stream);
+        }
+        ZKM_CUDA(cudaStreamSynchronize(c->stream));
+    }
+    std::lock_guard<std::mutex> rl(g->reg_mu);
+    const uint64_t h = g->next_handle++;
+    g->pks[h] = key;
+    return h;
+}
+
+static void g16_check(const G16Key& k, uint32_t log_n, size_t num_inputs, size_t num_aux) {
+    const int adicity = fr_two_adicity(k.curve);
+    if ((int)log_n > adicity) ZKM_FAIL(ZKM_ERR_DOMAIN, "log_n %u exceeds the two-adicity %d of Fr", log_n, adicity);
+    if (log_n > 28) ZKM_FAIL(ZKM_ERR_ARG, "log_n %u: witness maps above 2^28 are not supported by this build", log_n);
+    if (num_inputs + num_aux != k.m)
+        ZKM_FAIL(ZKM_ERR_ARG, "num_inputs + num_aux = %zu, but the key's a_query has %zu + 1 entries", num_inputs + num_aux, k.m);
+    if (k.reg[G16_L]->n != num_aux) ZKM_FAIL(ZKM_ERR_ARG, "num_aux = %zu, but the key's l_query has %zu entries", num_aux, k.reg[G16_L]->n);
+    if (k.reg[G16_H]->n > ((size_t)1 << log_n))
+        ZKM_FAIL(ZKM_ERR_ARG, "the key's h_query has %zu entries, more than the domain size 2^%u", k.reg[G16_H]->n, log_n);
+}
+
+// host buffers of zkm_groth16_prove: staged through the home lane's pinned and device workspaces
+struct G16Host {
+    const uint64_t *a, *b, *c, *assignment;
+    uint64_t *a_xy, *b_xy, *c_xy;
+    uint8_t *a_inf, *b_inf, *c_inf;
+};
+
+// One proof enqueued on `caller` (null: the home lane's stream) of device index `home`: witness map (h replaces b),
+// into_repr(h), the range check of the assignment, the five MSMs on lanes of their own (the b_g2 one joined only before
+// the G2 assembly), the G1 assembly (A, C), the G2 assembly (B).  All lanes are taken at once.
+static void g16_prove(const G16Key& k, int home, cudaStream_t caller, uint32_t log_n, size_t num_inputs, size_t num_aux,
+                      const uint64_t* r, const uint64_t* s, uint64_t* d_a, uint64_t* d_b, uint64_t* d_c, const uint64_t* d_asg,
+                      uint64_t* d_out, const G16Host* host) {
+    const int curve = k.curve;
+    const size_t S = (size_t)fr_words(curve), m = num_inputs + num_aux, nh = k.reg[G16_H]->n;
+    const size_t rw1 = 2 * (size_t)coord_words(curve, 1) + 1, rw2 = 2 * (size_t)coord_words(curve, 2) + 1;
+    const G16Ops ops = groth16_ops(curve);
+    std::vector<DevItem> items(5);
+    const size_t offs[5] = {0, 0, 0, 0, 0}, ns[5] = {nh, num_aux, m, m, m};
+    for (int i = 0; i < 5; i++) {
+        items[i].reg = k.reg[i];
+        items[i].offset = offs[i];
+        items[i].n = ns[i];
+    }
+    const ItemsPlan plan = plan_items(items, home);
+    MultiLaneGuard lanes(plan.devs, caller, &plan.keys);
+    Context* hc = lanes.c[0];
+    ZKM_CUDA(cudaSetDevice(hc->device));
+    if (!caller) caller = hc->stream;
+    StreamScope scope(hc, caller);
+    const size_t vb = (S * 8) << log_n, ab = m * S * 8;
+    if (host) {   // one pinned upload of a, b, c and the assignment
+        char* pin = (char*)hc->pin_in.get(3 * vb + ab);
+        memcpy(pin, host->a, vb);
+        memcpy(pin + vb, host->b, vb);
+        memcpy(pin + 2 * vb, host->c, vb);
+        if (ab) memcpy(pin + 3 * vb, host->assignment, ab);
+        char* d = (char*)hc->io_scalars.get(3 * vb + ab + 16);
+        h2d(d, pin, 3 * vb + ab, caller);
+        d_a = (uint64_t*)d;
+        d_b = (uint64_t*)(d + vb);
+        d_c = (uint64_t*)(d + 2 * vb);
+        d_asg = (const uint64_t*)(d + 3 * vb);
+    }
+    const size_t r1 = (rw1 * 8 + 15) & ~(size_t)15, r2 = (rw2 * 8 + 15) & ~(size_t)15, ob = (2 * rw1 + rw2) * 8;
+    char* w = (char*)hc->io_out.get(4 * r1 + r2 + 16 + (host ? ob : 0));
+    uint64_t* rec[5];
+    for (int i = 0; i < 5; i++) rec[i] = (uint64_t*)(w + i * r1);   // b_g2 last: its record may be the longer one
+    uint32_t* d_flag = (uint32_t*)(w + 4 * r1 + r2);
+    if (host) d_out = (uint64_t*)(w + 4 * r1 + r2 + 16);
+    ZKM_CUDA(cudaMemsetAsync(d_flag, 0, sizeof(uint32_t), caller));
+    witness_map_run(hc, curve, d_a, d_b, d_c, log_n, d_b, caller);
+    fr_into_repr_run(hc, curve, d_b, d_b, (uint64_t)nh, caller);
+    ops.range(hc, d_asg, m, d_flag, caller);
+    const uint64_t* scal[5] = {d_b, d_asg + num_inputs * S, d_asg, d_asg, d_asg};
+    for (int i = 0; i < 5; i++) {
+        items[i].d_scalars = scal[i];
+        items[i].d_out = rec[i];
+    }
+    // the G2 MSM is the longest: the G1 assembly (two ~SCALAR_BITS doubling chains) runs next to it
+    struct Join {
+        cudaStream_t s;
+        cudaEvent_t e = nullptr;
+        void now() {
+            if (!e) return;
+            cudaError_t rc = cudaStreamWaitEvent(s, e, 0);
+            cudaEventDestroy(e);
+            e = nullptr;
+            ZKM_CUDA(rc);
+        }
+        ~Join() {
+            try { now(); } catch (...) { cudaStreamSynchronize(s); cudaGetLastError(); }
+        }
+    } g2{caller};
+    items[G16_B2].done = &g2.e;
+    run_items(items, plan, lanes.c.data(), caller);
+    G16Args args;
+    memset(&args, 0, sizeof(args));
+    const G16Key::Dev& kd = k.dev[home];
+    args.key1 = kd.d_key;
+    args.key2 = kd.d_key + 5 * rw1;
+    for (int i = 0; i < 5; i++) {
+        args.rec[i] = rec[i];
+        args.rec_words[i] = (int)(i == G16_B2 ? rw2 : rw1);
+    }
+    args.range_flag = d_flag;
+    memcpy(args.r, r, S * 8);
+    memcpy(args.s, s, S * 8);
+    args.out = d_out;
+    ops.assemble(hc, 1, args, kd.d_tab1, caller);
+    g2.now();
+    ops.assemble(hc, 2, args, kd.d_tab2, caller);
+    if (!host) return;
+    uint64_t* h = (uint64_t*)hc->pin_out.get(ob);
+    ZKM_CUDA(cudaMemcpyAsync(h, d_out, ob, cudaMemcpyDeviceToHost, caller));
+    ZKM_CUDA(cudaStreamSynchronize(caller));
+    const uint64_t* ra = h;
+    const uint64_t* rb = h + rw1;
+    const uint64_t* rc = h + rw1 + rw2;
+    if (ra[rw1 - 1] == 2 || rb[rw2 - 1] == 2 || rc[rw1 - 1] == 2)
+        ZKM_FAIL(ZKM_ERR_SCALAR_RANGE, "an assignment element, r or s is not below the scalar modulus");
+    memcpy(host->a_xy, ra, (rw1 - 1) * 8);
+    memcpy(host->b_xy, rb, (rw2 - 1) * 8);
+    memcpy(host->c_xy, rc, (rw1 - 1) * 8);
+    *host->a_inf = ra[rw1 - 1] ? 1 : 0;
+    *host->b_inf = rb[rw2 - 1] ? 1 : 0;
+    *host->c_inf = rc[rw1 - 1] ? 1 : 0;
+}
+
 }  // namespace zkm
 
 using namespace zkm;
@@ -905,6 +1163,7 @@ void zkm_shutdown(void) {
     }
     {
         std::lock_guard<std::mutex> rl(og->reg_mu);
+        og->pks.clear();
         og->bases.clear();          // ~BasesReg frees the device memory
     }
     for (Shared* sh : og->devs) {
@@ -1451,6 +1710,55 @@ int32_t zkm_fixed_base_msm_device(int32_t curve, int32_t group, const uint64_t* 
         ZKM_CUDA(cudaSetDevice(c->device));
         StreamScope scope(c, s);
         fixed_base_run(c, curve, group, base_xy, base_inf != 0, d_scalars, n, d_out_xy, d_out_inf, nullptr, s);
+    });
+}
+
+int32_t zkm_groth16_pk_create(int32_t curve, const uint64_t* handles, const uint64_t* g1_xy, const uint8_t* g1_inf,
+                              const uint64_t* g2_xy, const uint8_t* g2_inf, uint64_t* pk_out) {
+    return guarded([&] {
+        if (!pk_out) ZKM_FAIL(ZKM_ERR_ARG, "null pk_out");
+        *pk_out = g16_create(curve, handles, g1_xy, g1_inf, g2_xy, g2_inf);
+    });
+}
+
+int32_t zkm_groth16_pk_release(uint64_t pk) {
+    return guarded([&] {
+        if (!g) ZKM_FAIL(ZKM_ERR_NOT_INIT, "zkm_init() has not been called (or failed)");
+        std::shared_ptr<G16Key> keep;     // destroyed (device memory freed) outside the registry lock
+        std::lock_guard<std::mutex> rl(g->reg_mu);
+        auto it = g->pks.find(pk);
+        if (it == g->pks.end()) ZKM_FAIL(ZKM_ERR_HANDLE, "unknown Groth16 proving key %llu", (unsigned long long)pk);
+        keep = std::move(it->second);
+        g->pks.erase(it);
+    });
+}
+
+int32_t zkm_groth16_prove(uint64_t pk, const uint64_t* a, const uint64_t* b, const uint64_t* c, uint32_t log_n,
+                          const uint64_t* assignment, size_t num_inputs, size_t num_aux, const uint64_t* r, const uint64_t* s,
+                          uint64_t* out_a_xy, uint8_t* out_a_inf, uint64_t* out_b_xy, uint8_t* out_b_inf, uint64_t* out_c_xy,
+                          uint8_t* out_c_inf) {
+    return guarded([&] {
+        if (!a || !b || !c || !r || !s || (num_inputs + num_aux && !assignment)) ZKM_FAIL(ZKM_ERR_ARG, "null pointer");
+        if (!out_a_xy || !out_a_inf || !out_b_xy || !out_b_inf || !out_c_xy || !out_c_inf) ZKM_FAIL(ZKM_ERR_ARG, "null output pointer");
+        std::shared_ptr<G16Key> key = g16_lookup(pk);
+        g16_check(*key, log_n, num_inputs, num_aux);
+        const G16Host host{a, b, c, assignment, out_a_xy, out_b_xy, out_c_xy, out_a_inf, out_b_inf, out_c_inf};
+        g16_prove(*key, pick_host_call_device(), nullptr, log_n, num_inputs, num_aux, r, s, nullptr, nullptr, nullptr, nullptr,
+                  nullptr, &host);
+    });
+}
+
+int32_t zkm_groth16_prove_device(uint64_t pk, uint64_t* d_a, uint64_t* d_b, uint64_t* d_c, uint32_t log_n,
+                                 const uint64_t* d_assignment, size_t num_inputs, size_t num_aux, const uint64_t* r,
+                                 const uint64_t* s, uint64_t* d_out, void* stream) {
+    return guarded([&] {
+        if (!d_a || !d_b || !d_c || !d_out || !r || !s || (num_inputs + num_aux && !d_assignment))
+            ZKM_FAIL(ZKM_ERR_ARG, "null pointer");
+        std::shared_ptr<G16Key> key = g16_lookup(pk);
+        g16_check(*key, log_n, num_inputs, num_aux);
+        const int home = home_device_of(d_out);
+        g16_prove(*key, home, call_stream(home, stream), log_n, num_inputs, num_aux, r, s, d_a, d_b, d_c, d_assignment, d_out,
+                  nullptr);
     });
 }
 

@@ -120,6 +120,41 @@ __global__ void __launch_bounds__(128) k_fb_columns(const char* __restrict__ wb_
     }
 }
 
+// sv B for a canonical scalar sv (SL 32-bit limbs) from the affine table of B (W rows of H entries, window c): signed
+// c-bit digits, one mixed addition per non-zero digit (a negative digit negates y), no doublings
+template <class F, int SL>
+__device__ __forceinline__ XYZZ<F> fb_table_mul(const uint32_t* sv, const char* __restrict__ table, int c, int W, uint32_t H) {
+    constexpr int CB = CoordIO<F>::BYTES;
+    const uint32_t mask = (1u << c) - 1u;
+    XYZZ<F> acc = XYZZ<F>::identity();
+    uint32_t s[SL + 2];   // indexed by window: kept in local memory, two loads per window
+    for (int k = 0; k < SL; k++) s[k] = sv[k];
+    s[SL] = 0;
+    s[SL + 1] = 0;
+    uint32_t carry = 0;
+    for (int w = 0; w < W; w++) {
+        const int lo = c * w;
+        const int li = lo >> 5, sh = lo & 31;
+        const uint64_t two = li < SL ? ((uint64_t)s[li] | ((uint64_t)s[li + 1] << 32)) : 0ull;
+        uint32_t d = (uint32_t)(two >> sh) & mask;
+        d += carry;
+        carry = 0;
+        uint32_t neg_d = 0;
+        if (d > H) {            // signed digit in [-H, H]: d - 2^c, carry one into the next window
+            d = (1u << c) - d;
+            neg_d = 1;
+            carry = 1;
+        }
+        if (d == 0) continue;
+        const char* p = table + ((size_t)w * H + (d - 1)) * 2 * CB;
+        const F x = CoordIO<F>::ld_gather(p);
+        F y = CoordIO<F>::ld_gather(p + CB);
+        if (neg_d) y = neg(y);
+        xyzz_madd(acc, x, y);
+    }
+    return acc;
+}
+
 // out[i] = s_i B from the affine table (W rows of H entries).  Scalars arrive in Montgomery form (upstream's
 // &[G::ScalarField]); `flag` (may be null) gets bit 0 when one is not < r.  base_inf: every output is the identity.
 template <class G>
@@ -129,8 +164,6 @@ k_fb_scalars(const uint32_t* __restrict__ scalars, uint64_t n, const char* __res
     typedef typename G::F F;
     typedef typename FbScalar<G>::P SP;
     constexpr int SL = SP::N;
-    constexpr int CB = CoordIO<F>::BYTES;
-    const uint32_t mask = (1u << c) - 1u;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
         Fp<SP> m = ld_fp<SP>(scalars + i * SL);
         if (flag) {   // canonical: m < r (top limb first)
@@ -143,31 +176,7 @@ k_fb_scalars(const uint32_t* __restrict__ scalars, uint64_t n, const char* __res
             Fp<SP> one_raw = Fp<SP>::zero();
             one_raw.l[0] = 1;   // a * 1 * R^-1 = into_repr(a)
             const Fp<SP> sv = fp_mul(m, one_raw);
-            uint32_t s[SL + 2];   // indexed by window: kept in local memory, two loads per window
-            for (int k = 0; k < SL; k++) s[k] = sv.l[k];
-            s[SL] = 0;
-            s[SL + 1] = 0;
-            uint32_t carry = 0;
-            for (int w = 0; w < W; w++) {
-                const int lo = c * w;
-                const int li = lo >> 5, sh = lo & 31;
-                const uint64_t two = li < SL ? ((uint64_t)s[li] | ((uint64_t)s[li + 1] << 32)) : 0ull;
-                uint32_t d = (uint32_t)(two >> sh) & mask;
-                d += carry;
-                carry = 0;
-                uint32_t neg_d = 0;
-                if (d > H) {            // signed digit in [-H, H]: d - 2^c, carry one into the next window
-                    d = (1u << c) - d;
-                    neg_d = 1;
-                    carry = 1;
-                }
-                if (d == 0) continue;
-                const char* p = table + ((size_t)w * H + (d - 1)) * 2 * CB;
-                const F x = CoordIO<F>::ld_gather(p);
-                F y = CoordIO<F>::ld_gather(p + CB);
-                if (neg_d) y = neg(y);
-                xyzz_madd(acc, x, y);
-            }
+            acc = fb_table_mul<F, SL>(sv.l, table, c, W, H);
         }
         st_xyzz(out + i, acc);
     }
@@ -195,6 +204,28 @@ inline int fixed_base_window_bits(int scalar_bits, size_t rec_bytes, size_t n) {
 template <class G>
 struct FixedBaseImpl {
     typedef typename G::F F;
+    static void normalize(Context* c, const XYZZ<F>* in, uint64_t m, char* out_xy, uint8_t* out_inf, cudaStream_t s) {
+        const uint64_t T = (m + FB_RUN - 1) / FB_RUN;
+        F* pre = (F*)c->ws[FB_WS_PRE].get(m * CoordIO<F>::BYTES);
+        ZKM_LAUNCH(k_fb_normalize<F>, (unsigned)((T + 127) / 128), 128, 0, s, in, m, T, pre, out_xy, out_inf);
+    }
+    // the affine table of a finite base (host record base_xy) for window cw: W rows of H entries, written to `table`
+    static void build_table(Context* c, const uint64_t* base_xy, int cw, int W, uint32_t H, char* table, cudaStream_t s) {
+        constexpr int CB = CoordIO<F>::BYTES;
+        constexpr size_t XB = sizeof(XYZZ<F>);
+        const size_t entries = (size_t)W * H;
+        FbBase b;
+        memcpy(b.w, base_xy, 2 * CB);
+        XYZZ<F>* wb = (XYZZ<F>*)c->ws[FB_WS_WB].get((size_t)W * (XB + 2 * CB));
+        char* wb_aff = (char*)(wb + W);
+        ZKM_LAUNCH(k_fb_window_bases<F>, 1, 32, 0, s, b, cw, W, wb);
+        normalize(c, wb, (uint64_t)W, wb_aff, nullptr, s);
+        const uint32_t m = H < FB_RUN ? H : FB_RUN;
+        const uint64_t threads = (uint64_t)W * (H / m);
+        XYZZ<F>* xyzz = (XYZZ<F>*)c->ws[FB_WS_XYZZ].get(entries * XB);
+        ZKM_LAUNCH(k_fb_columns<F>, (unsigned)((threads + 127) / 128), 128, 0, s, (const char*)wb_aff, W, H, m, xyzz);
+        normalize(c, xyzz, (uint64_t)entries, table, nullptr, s);
+    }
     // base: one affine record (host memory, 2 * CB bytes); d_flag: null, or a zeroed device word for the range check
     static void run(Context* c, const uint64_t* base_xy, bool base_inf, const uint64_t* d_scalars, size_t n, uint64_t* d_out_xy,
                     uint8_t* d_out_inf, uint32_t* d_flag, cudaStream_t s) {
@@ -207,29 +238,14 @@ struct FixedBaseImpl {
         const size_t entries = (size_t)W * H;
         char* table = (char*)c->ws[FB_WS_TAB].get(entries * 2 * CB);
         XYZZ<F>* xyzz = (XYZZ<F>*)c->ws[FB_WS_XYZZ].get((entries > n ? entries : n) * XB);
-        F* pre = (F*)c->ws[FB_WS_PRE].get((entries > n ? entries : n) * CB);
-        auto normalize = [&](const XYZZ<F>* in, uint64_t m, char* out_xy, uint8_t* out_inf) {
-            const uint64_t T = (m + FB_RUN - 1) / FB_RUN;
-            ZKM_LAUNCH(k_fb_normalize<F>, (unsigned)((T + 127) / 128), 128, 0, s, in, m, T, pre, out_xy, out_inf);
-        };
-        if (!base_inf) {
-            FbBase b;
-            memcpy(b.w, base_xy, 2 * CB);
-            XYZZ<F>* wb = (XYZZ<F>*)c->ws[FB_WS_WB].get((size_t)W * (XB + 2 * CB));
-            char* wb_aff = (char*)(wb + W);
-            ZKM_LAUNCH(k_fb_window_bases<F>, 1, 32, 0, s, b, cw, W, wb);
-            normalize(wb, (uint64_t)W, wb_aff, nullptr);
-            const uint32_t m = H < FB_RUN ? H : FB_RUN;
-            const uint64_t threads = (uint64_t)W * (H / m);
-            ZKM_LAUNCH(k_fb_columns<F>, (unsigned)((threads + 127) / 128), 128, 0, s, (const char*)wb_aff, W, H, m, xyzz);
-            normalize(xyzz, (uint64_t)entries, table, nullptr);
-        }
+        c->ws[FB_WS_PRE].get((entries > n ? entries : n) * CB);   // sized once for the table and the outputs
+        if (!base_inf) build_table(c, base_xy, cw, W, H, table, s);
         {
             const uint64_t blocks = (n + 127) / 128, cap = (uint64_t)c->sm_count * AccumMinBlocks<F>::value * 16;
             ZKM_LAUNCH(k_fb_scalars<G>, (unsigned)(blocks < cap ? blocks : cap), 128, 0, s, (const uint32_t*)d_scalars, (uint64_t)n,
                        (const char*)table, cw, W, H, base_inf ? 1 : 0, xyzz, d_flag);
         }
-        normalize(xyzz, (uint64_t)n, (char*)d_out_xy, d_out_inf);
+        normalize(c, xyzz, (uint64_t)n, (char*)d_out_xy, d_out_inf, s);
     }
 };
 

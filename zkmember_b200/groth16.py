@@ -10,8 +10,9 @@ and this runs the seven NTTs and the pointwise step on the GPU without leaving H
 (src/prover.rs: h_query, l_query, a_query, b_g1_query on G1, b_g2_query on G2).
 
 `ProvingKey` + `create_proof` mirror `create_proof_with_reduction_and_matrices` from the witness map to the
-`Proof { a, b, c }` (final assembly included: `calculate_coeff`, g_c = s g_a + r g1_b - rs delta + l_aux + h_acc),
-and `serialize.Proof.serialize()` gives the 192-byte (BLS12-381) arkworks wire format.
+`Proof { a, b, c }` (final assembly included: `calculate_coeff`, g_c = s g_a + r g1_b - rs delta + l_aux + h_acc) as ONE
+library call (`zkm_groth16_prove`): witness map, the five MSMs and the assembly stay on the device.
+`serialize.Proof.serialize()` gives the 192-byte (BLS12-381) arkworks wire format.
 """
 from __future__ import annotations
 
@@ -20,7 +21,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from .msm import RegisteredBases, AffinePoint, VariableBaseMSM, FR_WORDS, coord_words, _curve_id
+from .msm import RegisteredBases, AffinePoint, FR_WORDS, coord_words, _curve_id, _ptr
 from .serialize import Proof, FR_MODULUS
 
 
@@ -86,7 +87,8 @@ def _scalar_limbs(curve: int, v: int) -> np.ndarray:
 class ProvingKey:
     """ark_groth16::ProvingKey: the verifying-key elements the prover touches plus the five query vectors.
     `a_query`, `b_g1_query`, `b_g2_query` are the FULL vectors (entry 0 belongs to the constant-one variable and is
-    added outside the MSM, as `calculate_coeff` does); the remaining entries are registered on the device once."""
+    added outside the MSM, as `calculate_coeff` does); the remaining entries are registered on the device once, and
+    the device key (`handle`, zkm_groth16_pk_create) refers to those registrations and the key's eight points."""
 
     def __init__(self, curve, alpha_g1, beta_g1, beta_g2, delta_g1, delta_g2, a_query, b_g1_query, b_g2_query,
                  h_query, l_query, infinity=None, precompute=True):
@@ -107,47 +109,67 @@ class ProvingKey:
         self.msms = ProvingKeyMSMs(self.curve, h_query, l_query, a_query[1:], b_g1_query[1:], b_g2_query[1:],
                                    infinity={"h": flags["h"], "l": flags["l"], "a": tail["a"], "b_g1": tail["b_g1"],
                                              "b_g2": tail["b_g2"]}, precompute=precompute)
+        self.num_vars = len(a_query) - 1
+        self.num_aux = self.msms.l.n
+        ms = self.msms
+        handles = np.array([ms.h.handle, ms.l.handle, ms.a.handle, ms.b_g1.handle, ms.b_g2.handle], dtype=np.uint64)
+        g1 = np.ascontiguousarray(np.stack([self.alpha_g1, self.beta_g1, self.delta_g1, self.first["a"][0],
+                                            self.first["b_g1"][0]]))
+        g1_inf = np.array([0, 0, 0, self.first["a"][1], self.first["b_g1"][1]], dtype=np.uint8)
+        g2 = np.ascontiguousarray(np.stack([self.beta_g2, self.delta_g2, self.first["b_g2"][0]]))
+        g2_inf = np.array([0, 0, self.first["b_g2"][1]], dtype=np.uint8)
+        h = ctypes.c_uint64(0)
+        try:
+            _lib.check(_lib.lib().zkm_groth16_pk_create(self.curve, _ptr(handles), _ptr(g1), _ptr(g1_inf), _ptr(g2),
+                                                        _ptr(g2_inf), ctypes.byref(h)))
+        except Exception:
+            self.msms.release()
+            raise
+        self.handle = h.value
 
     def release(self):
+        if self.handle:
+            _lib.check(_lib.lib().zkm_groth16_pk_release(self.handle))
+            self.handle = 0
         self.msms.release()
 
-
-def _lincomb(curve: int, group: int, terms) -> AffinePoint:
-    """sum of k_i * P_i for a handful of (xy limbs, infinity, int scalar) terms -- a tiny MSM through the same C ABI."""
-    xy = np.stack([t[0] for t in terms])
-    inf = np.array([1 if t[1] else 0 for t in terms], dtype=np.uint8)
-    sc = np.stack([_scalar_limbs(curve, t[2] % FR_MODULUS[curve]) for t in terms])
-    return VariableBaseMSM.multi_scalar_mul(xy, sc, curve=curve, group=group, infinity=inf)
+    def prove_device(self, d_a: int, d_b: int, d_c: int, log_n: int, d_assignment: int, num_inputs: int, r: int, s: int,
+                     d_out: int, stream: int = 0):
+        """Device form of `create_proof` (zkm_groth16_prove_device): d_a, d_b, d_c (2^log_n Montgomery Fr each, consumed)
+        and d_assignment (num_inputs + num_aux canonical scalars) are device pointers; d_out receives the records A, B,
+        C (2 W1 + 1, 2 W2 + 1, 2 W1 + 1 words; last word 0 finite, 1 infinity, 2 invalid scalar).  Enqueued on `stream`
+        without a host wait; r and s are reduced modulo the scalar modulus."""
+        rl, sl = (_scalar_limbs(self.curve, v % FR_MODULUS[self.curve]) for v in (r, s))
+        _lib.check(_lib.lib().zkm_groth16_prove_device(
+            self.handle, ctypes.c_void_p(d_a), ctypes.c_void_p(d_b), ctypes.c_void_p(d_c), int(log_n),
+            ctypes.c_void_p(d_assignment), int(num_inputs), self.num_vars - int(num_inputs), _ptr(rl), _ptr(sl),
+            ctypes.c_void_p(d_out), ctypes.c_void_p(stream)))
 
 
 def create_proof(pk: ProvingKey, r: int, s: int, a, b, c, input_assignment, aux_assignment) -> Proof:
     """ark_groth16::create_proof_with_reduction_and_matrices (ark-groth16 0.3.0 src/prover.rs) after constraint
     synthesis: `a`, `b`, `c` are the evaluation vectors handed to the witness map (Montgomery Fr, domain size n),
     `input_assignment` (without the leading one) and `aux_assignment` the canonical (`into_repr`) assignments,
-    r and s the prover's blinding scalars."""
-    from .kzg import KZG10
+    r and s the prover's blinding scalars (reduced modulo the scalar modulus)."""
     curve = pk.curve
     S = FR_WORDS[curve]
-    h = witness_map(a, b, c, curve=curve)
-    n = len(h)
+    a = np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, S)
+    b = np.ascontiguousarray(b, dtype=np.uint64).reshape(-1, S)
+    c = np.ascontiguousarray(c, dtype=np.uint64).reshape(-1, S)
+    n = len(a)
+    log_n = n.bit_length() - 1
+    if n == 0 or (1 << log_n) != n or len(b) != n or len(c) != n:
+        raise ValueError("a, b, c must have the same power-of-two length")
     inputs = np.ascontiguousarray(input_assignment, dtype=np.uint64).reshape(-1, S)
     aux = np.ascontiguousarray(aux_assignment, dtype=np.uint64).reshape(-1, S)
-    full = np.concatenate([inputs, aux])
-    # h_acc = MSM(h_query, h[..n-1].into_repr()): into_repr + MSM on the device (the commit entry point does both)
-    h_acc = KZG10.commit(pk.msms.h, h[:n - 1])
-    l_acc = pk.msms.l.msm(aux)
-    a_acc = pk.msms.a.msm(full)
-    b1_acc = pk.msms.b_g1.msm(full)
-    b2_acc = pk.msms.b_g2.msm(full)
-    one = 1
-    # calculate_coeff(initial, query, vk_param, assignment) = initial + query[0] + MSM(query[1..], assignment) + vk_param
-    g_a = _lincomb(curve, 1, [(pk.delta_g1, False, r), (pk.first["a"][0], pk.first["a"][1], one),
-                              (a_acc.xy, a_acc.infinity, one), (pk.alpha_g1, False, one)])
-    g1_b = _lincomb(curve, 1, [(pk.delta_g1, False, s), (pk.first["b_g1"][0], pk.first["b_g1"][1], one),
-                               (b1_acc.xy, b1_acc.infinity, one), (pk.beta_g1, False, one)])
-    g2_b = _lincomb(curve, 2, [(pk.delta_g2, False, s), (pk.first["b_g2"][0], pk.first["b_g2"][1], one),
-                               (b2_acc.xy, b2_acc.infinity, one), (pk.beta_g2, False, one)])
-    # g_c = s g_a + r g1_b - (r s) delta_g1 + l_aux_acc + h_acc
-    g_c = _lincomb(curve, 1, [(g_a.xy, g_a.infinity, s), (g1_b.xy, g1_b.infinity, r), (pk.delta_g1, False, -(r * s)),
-                              (l_acc.xy, l_acc.infinity, one), (h_acc.xy, h_acc.infinity, one)])
-    return Proof(a=g_a, b=g2_b, c=g_c)
+    full = np.ascontiguousarray(np.concatenate([inputs, aux]))
+    rl, sl = (_scalar_limbs(curve, v % FR_MODULUS[curve]) for v in (r, s))
+    W1, W2 = coord_words(curve, 1), coord_words(curve, 2)
+    axy, bxy, cxy = np.zeros(2 * W1, dtype=np.uint64), np.zeros(2 * W2, dtype=np.uint64), np.zeros(2 * W1, dtype=np.uint64)
+    inf = np.zeros(3, dtype=np.uint8)
+    p = lambda x: ctypes.c_void_p(x.ctypes.data)
+    _lib.check(_lib.lib().zkm_groth16_prove(pk.handle, p(a), p(b), p(c), log_n, _ptr(full), len(inputs), len(aux), p(rl),
+                                            p(sl), p(axy), ctypes.c_void_p(inf.ctypes.data), p(bxy),
+                                            ctypes.c_void_p(inf.ctypes.data + 1), p(cxy), ctypes.c_void_p(inf.ctypes.data + 2)))
+    return Proof(a=AffinePoint(curve, 1, axy, bool(inf[0])), b=AffinePoint(curve, 2, bxy, bool(inf[1])),
+                 c=AffinePoint(curve, 1, cxy, bool(inf[2])))
