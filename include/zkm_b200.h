@@ -149,6 +149,45 @@ int32_t zkm_kzg_open(uint64_t handle_g, uint64_t handle_gamma_g, const uint64_t*
                      const uint64_t* blinding_coeffs, size_t nb, const uint64_t* point, uint64_t* out_w_xy,
                      uint8_t* out_w_inf, uint64_t* out_random_v);
 
+/* ---- batch commitments and openings (MarlinKZG10) --------------------------------------------------
+ * The group side of ark-poly-commit 0.3.0 MarlinKZG10::{commit, batch_open, open_combinations} (src/marlin/marlin_pc).
+ * The MarlinKZG10 bookkeeping (opening-challenge counter, degree-bound shifts, linear combinations) stays with the
+ * caller; these calls take flat lists.  Polynomials are Montgomery Fr coefficients, low degree first.
+ *
+ * zkm_kzg_commit_many: item i = MSM(powers_of_g[shift_i + z_i ..], coeffs_i[z_i ..]) with z_i its leading zero
+ * coefficients, plus MSM(powers_of_gamma_g, blind_i) when nb_i > 0 (blind / nb may be NULL: no hiding).  A Marlin
+ * polynomial with a degree bound d is two items, the second with shift D - d.  All MSMs run concurrently, the sums are
+ * formed on the device, one read-back.  At most 23 items.  out_xy: count x 2 W words, out_inf: count flags.
+ * n_i counts every coefficient given, trailing zeros included: pass the polynomial without them (as DensePolynomial
+ * keeps it) so that a bounded polynomial of degree d fits shift D - d.
+ * Errors: ZKM_ERR_HANDLE when shift_i + n_i exceeds powers_of_g or nb_i exceeds powers_of_gamma_g. */
+int32_t zkm_kzg_commit_many(uint64_t handle_g, uint64_t handle_gamma_g, int32_t count, const uint64_t* const* coeffs,
+                            const size_t* n, const size_t* shift, const uint64_t* const* blind, const size_t* nb,
+                            uint64_t* out_xy, uint8_t* out_inf);
+/* zkm_kzg_open_batch: opening proofs at npoints points (at most 23).  Term t names a point, a polynomial, a blinding
+ * polynomial (-1: none), a shift s_t and a Montgomery Fr coefficient c_t (term_coeff: nterms x S words).  Per point i:
+ *   W_i        = commit_g(sum_t c_t X^(s_t) q_(poly_t, z_i)) + commit_gamma_g(sum_t c_t q_(blind_t, z_i))
+ *   random_v_i = sum_t c_t blind_t(z_i)                 q_(p, z) = (p(X) - p(z)) / (X - z)
+ * and out_evals[t] = poly_t(z_(point_t)) (Montgomery; out_evals may be NULL).  out_w_xy: npoints x 2 W words,
+ * out_w_inf: npoints flags, out_random_v: npoints x S words.  At most 65535 terms.  One pinned upload and one read-back.
+ * Errors: ZKM_ERR_ARG for an index out of range, null arrays, a G2 or other-curve registration; ZKM_ERR_HANDLE when
+ * s_t + n - 1 exceeds powers_of_g or nb - 1 exceeds powers_of_gamma_g, or for a released handle. */
+int32_t zkm_kzg_open_batch(uint64_t handle_g, uint64_t handle_gamma_g, int32_t npolys, const uint64_t* const* coeffs,
+                           const size_t* n, int32_t nblind, const uint64_t* const* blind, const size_t* nb, int32_t npoints,
+                           const uint64_t* points, int32_t nterms, const int32_t* term_point, const int32_t* term_poly,
+                           const int32_t* term_blind, const size_t* term_shift, const uint64_t* term_coeff,
+                           uint64_t* out_w_xy, uint8_t* out_w_inf, uint64_t* out_random_v, uint64_t* out_evals);
+/* The same with the polynomials (d_coeffs[i], d_blind[i]: 16-byte aligned, ZKM_ERR_ARG otherwise) and the outputs in
+ * device memory of one device (the device of d_out_w; a polynomial elsewhere is ZKM_ERR_ARG): d_out_w receives npoints records of 2 W + 1 words (flag word 0 finite, 1 infinity), d_out_random_v npoints x S
+ * words, d_out_evals (may be NULL) nterms x S words.  The index arrays, points and term coefficients stay HOST arrays.
+ * A fixed launch sequence on `stream` (NULL: the library's stream of that device); no read-back, no host wait. */
+int32_t zkm_kzg_open_batch_device(uint64_t handle_g, uint64_t handle_gamma_g, int32_t npolys, const uint64_t* const* d_coeffs,
+                                  const size_t* n, int32_t nblind, const uint64_t* const* d_blind, const size_t* nb,
+                                  int32_t npoints, const uint64_t* points, int32_t nterms, const int32_t* term_point,
+                                  const int32_t* term_poly, const int32_t* term_blind, const size_t* term_shift,
+                                  const uint64_t* term_coeff, uint64_t* d_out_w, uint64_t* d_out_random_v,
+                                  uint64_t* d_out_evals, void* stream);
+
 /* ---- fixed-base batch scalar multiplication -------------------------------------------------------
  * Replaces ark_ec::msm::FixedBaseMSM::{get_window_table, multi_scalar_mul} (ark-ec 0.3.0 src/msm/fixed_base.rs)
  * + batch_normalization_into_affine: the queries of Groth16::circuit_specific_setup (ark-groth16 0.3.0

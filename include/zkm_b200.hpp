@@ -12,6 +12,7 @@
 //   zkm::ProvingKeyBases / KZG10::commit                        registered bases (pk / SRS reuse)
 //   zkm::serialize(point) / zkm::Proof<Curve>::serialize()      arkworks' compressed CanonicalSerialize (host code)
 //   zkm::Groth16ProvingKey<Curve> / zkm::create_proof            ark-groth16 0.3.0 src/prover.rs (after synthesis)
+//   zkm::MarlinKZG10::{commit, batch_open}                      ark-poly-commit 0.3.0 src/marlin/marlin_pc (group side)
 //
 // Types are plain structs with arkworks' memory layout: Fp256 = 4 x u64 Montgomery limbs, Fp384 = 6,
 // BigInteger256 = 4 x u64 canonical limbs (BigInteger384 = 6 for BW6-761), GroupAffine{x, y, infinity}.  Errors of the C ABI become
@@ -334,6 +335,103 @@ struct KZG10 {
               "zkm_kzg_open");
         pr.w = detail::unpack<Curve, 1>(out, out_inf);
         return pr;
+    }
+};
+
+// ark_poly_commit::marlin_pc (0.3.0 src/marlin/marlin_pc/mod.rs), the group side: commitments with degree-bound shifts
+// and batch openings over flat lists (zkm_kzg_commit_many / zkm_kzg_open_batch).  The MarlinKZG10 bookkeeping (opening
+// challenge powers, shifts D - d, linear combinations) is the caller's, as in the Python layer.
+template <class Curve>
+struct MarlinCommitItem {      // MSM(powers_of_g[shift + zeros ..], coeffs) + MSM(powers_of_gamma_g, blind)
+    const std::vector<typename Curve::Fr>* coeffs;
+    size_t shift;
+    const std::vector<typename Curve::Fr>* blind;   // null or empty: no hiding term
+};
+template <class Curve>
+struct MarlinTerm {            // c X^shift q_(polys[poly], points[point]) [+ c q_(blinds[blind], z)]
+    int32_t point, poly, blind;   // blind = -1: none
+    size_t shift;
+    typename Curve::Fr coeff;
+};
+template <class Curve>
+struct MarlinBatchProof {      // one kzg10::Proof per point, and poly_t(z_t) per term
+    std::vector<KZGProof<Curve>> proofs;
+    std::vector<typename Curve::Fr> evals;
+};
+struct MarlinKZG10 {
+    // coefficients up to the top non-zero one (DensePolynomial drops trailing zeros; the C ABI's bound checks count
+    // every coefficient it is given)
+    template <class F>
+    static size_t trimmed_size(const std::vector<F>& p) {
+        size_t n = p.size();
+        F zero;
+        std::memset(&zero, 0, sizeof(zero));
+        while (n && p[n - 1] == zero) n--;
+        return n;
+    }
+    template <class Curve>
+    static std::vector<G1Affine<Curve>> commit(const RegisteredBases<Curve, 1>& powers_of_g, const RegisteredBases<Curve, 1>* powers_of_gamma_g,
+                                               const std::vector<MarlinCommitItem<Curve>>& items) {
+        const size_t k = items.size(), W2 = 2 * sizeof(typename Curve::Fq) / 8;
+        std::vector<const uint64_t*> cp(k), bp(k);
+        std::vector<size_t> n(k), sh(k), nb(k);
+        for (size_t i = 0; i < k; i++) {
+            cp[i] = reinterpret_cast<const uint64_t*>(items[i].coeffs->data());
+            n[i] = trimmed_size(*items[i].coeffs);
+            sh[i] = items[i].shift;
+            bp[i] = items[i].blind ? reinterpret_cast<const uint64_t*>(items[i].blind->data()) : nullptr;
+            nb[i] = items[i].blind ? items[i].blind->size() : 0;
+        }
+        std::vector<uint64_t> out(std::max<size_t>(k, 1) * W2);
+        std::vector<uint8_t> inf(std::max<size_t>(k, 1));
+        check(zkm_kzg_commit_many(powers_of_g.handle(), powers_of_gamma_g ? powers_of_gamma_g->handle() : 0, (int32_t)k, cp.data(), n.data(),
+                                  sh.data(), bp.data(), nb.data(), out.data(), inf.data()),
+              "zkm_kzg_commit_many");
+        std::vector<G1Affine<Curve>> res;
+        for (size_t i = 0; i < k; i++)
+            res.push_back(detail::unpack<Curve, 1>(std::vector<uint64_t>(out.begin() + i * W2, out.begin() + (i + 1) * W2), inf[i]));
+        return res;
+    }
+    template <class Curve>
+    static MarlinBatchProof<Curve> batch_open(const RegisteredBases<Curve, 1>& powers_of_g, const RegisteredBases<Curve, 1>* powers_of_gamma_g,
+                                              const std::vector<const std::vector<typename Curve::Fr>*>& polys,
+                                              const std::vector<const std::vector<typename Curve::Fr>*>& blinds,
+                                              const std::vector<typename Curve::Fr>& points, const std::vector<MarlinTerm<Curve>>& terms) {
+        typedef typename Curve::Fr F;
+        const size_t W2 = 2 * sizeof(typename Curve::Fq) / 8, np = points.size(), nt = terms.size();
+        std::vector<const uint64_t*> cp, bp;
+        std::vector<size_t> n, nb, ts;
+        for (auto* p : polys) { cp.push_back(reinterpret_cast<const uint64_t*>(p->data())); n.push_back(trimmed_size(*p)); }
+        for (auto* b : blinds) { bp.push_back(reinterpret_cast<const uint64_t*>(b->data())); nb.push_back(b->size()); }
+        std::vector<int32_t> tp, tq, tb;
+        std::vector<F> tc;
+        for (const auto& t : terms) {
+            tp.push_back(t.point);
+            tq.push_back(t.poly);
+            tb.push_back(t.blind);
+            ts.push_back(t.shift);
+            tc.push_back(t.coeff);
+        }
+        std::vector<uint64_t> w(std::max<size_t>(np, 1) * W2);
+        std::vector<uint8_t> winf(std::max<size_t>(np, 1));
+        MarlinBatchProof<Curve> res;
+        std::vector<F> rv(std::max<size_t>(np, 1));
+        res.evals.resize(nt);
+        check(zkm_kzg_open_batch(powers_of_g.handle(), powers_of_gamma_g ? powers_of_gamma_g->handle() : 0, (int32_t)polys.size(), cp.data(),
+                                 n.data(), (int32_t)blinds.size(), bp.data(), nb.data(), (int32_t)np,
+                                 reinterpret_cast<const uint64_t*>(points.data()), (int32_t)nt, tp.data(), tq.data(), tb.data(), ts.data(),
+                                 reinterpret_cast<const uint64_t*>(tc.data()), w.data(), winf.data(), reinterpret_cast<uint64_t*>(rv.data()),
+                                 reinterpret_cast<uint64_t*>(res.evals.data())),
+              "zkm_kzg_open_batch");
+        for (size_t i = 0; i < np; i++) {
+            KZGProof<Curve> pr;
+            pr.w = detail::unpack<Curve, 1>(std::vector<uint64_t>(w.begin() + i * W2, w.begin() + (i + 1) * W2), winf[i]);
+            pr.hiding = false;
+            for (const auto& t : terms) pr.hiding = pr.hiding || (t.point == (int32_t)i && t.blind >= 0);
+            pr.random_v = rv[i];
+            res.proofs.push_back(pr);
+        }
+        return res;
     }
 };
 

@@ -59,6 +59,20 @@ extern "C" {
     pub fn zkm_groth16_prove_device(pk: u64, d_a: *mut u64, d_b: *mut u64, d_c: *mut u64, log_n: u32,
                                     d_assignment: *const u64, num_inputs: usize, num_aux: usize, r: *const u64,
                                     s: *const u64, d_out: *mut u64, stream: *mut c_void) -> i32;
+    pub fn zkm_kzg_commit_many(handle_g: u64, handle_gamma_g: u64, count: i32, coeffs: *const *const u64, n: *const usize,
+                               shift: *const usize, blind: *const *const u64, nb: *const usize, out_xy: *mut u64,
+                               out_inf: *mut u8) -> i32;
+    pub fn zkm_kzg_open_batch(handle_g: u64, handle_gamma_g: u64, npolys: i32, coeffs: *const *const u64, n: *const usize,
+                              nblind: i32, blind: *const *const u64, nb: *const usize, npoints: i32, points: *const u64,
+                              nterms: i32, term_point: *const i32, term_poly: *const i32, term_blind: *const i32,
+                              term_shift: *const usize, term_coeff: *const u64, out_w_xy: *mut u64, out_w_inf: *mut u8,
+                              out_random_v: *mut u64, out_evals: *mut u64) -> i32;
+    pub fn zkm_kzg_open_batch_device(handle_g: u64, handle_gamma_g: u64, npolys: i32, d_coeffs: *const *const u64,
+                                     n: *const usize, nblind: i32, d_blind: *const *const u64, nb: *const usize, npoints: i32,
+                                     points: *const u64, nterms: i32, term_point: *const i32, term_poly: *const i32,
+                                     term_blind: *const i32, term_shift: *const usize, term_coeff: *const u64,
+                                     d_out_w: *mut u64, d_out_random_v: *mut u64, d_out_evals: *mut u64,
+                                     stream: *mut c_void) -> i32;
 }
 
 /// Panics with the library's message: the upstream functions are infallible and there is deliberately

@@ -35,6 +35,7 @@ SYMBOLS = [
     "zkm_kzg_commit_hiding", "zkm_kzg_open", "zkm_profile_last_msm_counts", "zkm_msm_cache_clear", "zkm_msm_cache_stats",
     "zkm_fixed_base_msm", "zkm_fixed_base_msm_device",
     "zkm_groth16_pk_create", "zkm_groth16_pk_release", "zkm_groth16_prove", "zkm_groth16_prove_device",
+    "zkm_kzg_commit_many", "zkm_kzg_open_batch", "zkm_kzg_open_batch_device",
 ]
 
 # zkm_bases_register_ex flags (include/zkm_b200.h)
@@ -114,6 +115,11 @@ def load():
     L.zkm_groth16_pk_release.argtypes = [u64]
     L.zkm_groth16_prove.argtypes = [u64, u64p, u64p, u64p, u32, u64p, sz, sz, u64p, u64p, u64p, u8p, u64p, u8p, u64p, u8p]
     L.zkm_groth16_prove_device.argtypes = [u64, u64p, u64p, u64p, u32, u64p, sz, sz, u64p, u64p, u64p, vp]
+    L.zkm_kzg_commit_many.argtypes = [u64, u64, i32, vp, vp, vp, vp, vp, u64p, u8p]
+    L.zkm_kzg_open_batch.argtypes = [u64, u64, i32, vp, vp, i32, vp, vp, i32, u64p, i32, vp, vp, vp, vp, u64p, u64p, u8p, u64p,
+                                     u64p]
+    L.zkm_kzg_open_batch_device.argtypes = [u64, u64, i32, vp, vp, i32, vp, vp, i32, u64p, i32, vp, vp, vp, vp, u64p, u64p, u64p,
+                                            u64p, vp]
     _lib = L
     return L
 

@@ -9,6 +9,7 @@
 
 #include "zkm_common.cuh"
 #include "zkm_groth16_ops.cuh"
+#include "zkm_kzg_ops.cuh"
 
 namespace zkm {
 
@@ -1401,6 +1402,365 @@ int32_t zkm_kzg_open(uint64_t handle_g, uint64_t handle_gamma_g, const uint64_t*
             throw ZkmError{rc2};
         }
         add_two_points(rg->curve, 1, w_xy.data(), w_inf, h_xy.data(), h_inf, out_w_xy, out_w_inf);
+    });
+}
+
+// ------------------------------------------------------------------------------------------ MarlinKZG10 batch calls
+// MSM outputs are 16-byte aligned slots (k_msm_final writes with 128-bit stores); k_points_sum reads packed records.
+// Every output is the sum of two records (the hiding one the identity when there is none): the slots are packed with
+// one 2D copy and each pair is summed into an aligned slot of `sums`.
+static void sum_record_pairs(Context* hc, int curve, const char* slots, size_t nout, char* packed, char* sums, cudaStream_t s) {
+    const size_t rb = rec_bytes(curve, 1), r1 = (rb + 15) & ~(size_t)15;
+    if (nout == 0) return;
+    ZKM_CUDA(cudaMemcpy2DAsync(packed, rb, slots, r1, rb, 2 * nout, cudaMemcpyDeviceToDevice, s));
+    for (size_t i = 0; i < nout; i++)
+        points_sum_run(hc, curve, 1, (const uint64_t*)(packed + 2 * i * rb), 2, (uint64_t*)(sums + i * r1), s);
+}
+
+static std::shared_ptr<BasesReg> kzg_powers(uint64_t handle, int curve, const char* what) {
+    std::shared_ptr<BasesReg> r = lookup(handle, 0, 0);
+    if (r->group != 1 || (curve >= 0 && r->curve != curve)) ZKM_FAIL(ZKM_ERR_ARG, "%s must be G1 bases of the curve of powers_of_g", what);
+    return r;
+}
+
+static void kzg_commit_many_impl(uint64_t handle_g, uint64_t handle_gamma_g, int32_t count, const uint64_t* const* coeffs,
+                                 const size_t* n, const size_t* shift, const uint64_t* const* blind, const size_t* nb,
+                                 uint64_t* out_xy, uint8_t* out_inf) {
+    std::shared_ptr<BasesReg> rg = kzg_powers(handle_g, -1, "powers_of_g");
+    if (count < 0 || 2 * count > ZKM_NUM_LANES - 2) ZKM_FAIL(ZKM_ERR_ARG, "count must be 0..%d", (ZKM_NUM_LANES - 2) / 2);
+    if (count && (!coeffs || !n || !shift || !out_xy || !out_inf)) ZKM_FAIL(ZKM_ERR_ARG, "null argument array");
+    if (!blind != !nb) ZKM_FAIL(ZKM_ERR_ARG, "blind and nb must both be given or both be NULL");
+    const int curve = rg->curve;
+    const size_t S = (size_t)fr_words(curve), sb = S * 8, W2 = 2 * (size_t)coord_words(curve, 1);
+    std::shared_ptr<BasesReg> rh;
+    std::vector<size_t> zeros(count), off(count), boff(count);
+    size_t total = 0;
+    for (int i = 0; i < count; i++) {
+        if (n[i] && !coeffs[i]) ZKM_FAIL(ZKM_ERR_ARG, "item %d: null coefficients", i);
+        if (shift[i] > rg->n || n[i] > rg->n - shift[i])
+            ZKM_FAIL(ZKM_ERR_HANDLE, "item %d: shift %zu + %zu coefficients exceed the %zu registered powers", i, shift[i], n[i], rg->n);
+        zeros[i] = leading_zero_coeffs(coeffs[i], n[i], S);
+        off[i] = total;
+        total += n[i] - zeros[i];
+    }
+    for (int i = 0; i < count; i++) {
+        const size_t k = nb ? nb[i] : 0;
+        if (k && !rh) rh = kzg_powers(handle_gamma_g, curve, "powers_of_gamma_g");
+        if (k && !blind[i]) ZKM_FAIL(ZKM_ERR_ARG, "item %d: null blinding polynomial", i);
+        if (k > (rh ? rh->n : 0)) ZKM_FAIL(ZKM_ERR_HANDLE, "item %d: %zu blinding coefficients exceed powers_of_gamma_g", i, k);
+        boff[i] = total;
+        total += k;
+    }
+    if (count == 0) return;
+    std::vector<DevItem> items(2 * count);
+    for (int i = 0; i < count; i++) {
+        const size_t k = nb ? nb[i] : 0;
+        items[2 * i].reg = rg;
+        items[2 * i].offset = n[i] - zeros[i] ? shift[i] + zeros[i] : 0;
+        items[2 * i].n = n[i] - zeros[i];
+        items[2 * i + 1].reg = k ? rh : rg;
+        items[2 * i + 1].offset = 0;
+        items[2 * i + 1].n = k;
+    }
+    const int home = rg->parts[0].dev;
+    const ItemsPlan plan = plan_items(items, home);
+    MultiLaneGuard lanes(plan.devs, nullptr, &plan.keys);
+    Context* hc = lanes.c[0];
+    ZKM_CUDA(cudaSetDevice(hc->device));
+    cudaStream_t s = hc->stream;
+    StreamScope scope(hc, s);
+    char* pin = (char*)hc->pin_in.get(total * sb + 16);
+    for (int i = 0; i < count; i++) {
+        memcpy(pin + off[i] * sb, coeffs[i] + zeros[i] * S, (n[i] - zeros[i]) * sb);
+        if (nb && nb[i]) memcpy(pin + boff[i] * sb, blind[i], nb[i] * sb);
+    }
+    char* d = (char*)hc->io_scalars.get(total * sb + 16);
+    h2d(d, pin, total * sb, s);
+    fr_into_repr_run(hc, curve, (const uint64_t*)d, (uint64_t*)d, (uint64_t)total, s);   // convert_to_bigints
+    const size_t rb = rec_bytes(curve, 1), r1 = (rb + 15) & ~(size_t)15;
+    char* o = (char*)hc->io_out.get(2 * count * r1 + 2 * count * rb + count * r1 + 32);
+    char* slots = o;
+    char* packed = o + 2 * count * r1;
+    char* sums = packed + ((2 * count * rb + 15) & ~(size_t)15);
+    for (int i = 0; i < count; i++) {
+        items[2 * i].d_scalars = (const uint64_t*)(d + off[i] * sb);
+        items[2 * i].d_out = (uint64_t*)(slots + 2 * i * r1);
+        items[2 * i + 1].d_scalars = (const uint64_t*)(d + boff[i] * sb);
+        items[2 * i + 1].d_out = (uint64_t*)(slots + (2 * i + 1) * r1);
+    }
+    run_items(items, plan, lanes.c.data(), s);
+    sum_record_pairs(hc, curve, slots, count, packed, sums, s);
+    uint64_t* h = (uint64_t*)hc->pin_out.get(count * r1);
+    ZKM_CUDA(cudaMemcpyAsync(h, sums, count * r1, cudaMemcpyDeviceToHost, s));
+    ZKM_CUDA(cudaStreamSynchronize(s));
+    for (int i = 0; i < count; i++) {
+        const uint64_t* rec = (const uint64_t*)((const char*)h + i * r1);
+        memcpy(out_xy + i * W2, rec, W2 * 8);
+        out_inf[i] = rec_flag(rec[W2]);
+    }
+}
+
+// The arguments of zkm_kzg_open_batch[_device]; coeffs / blind are host or device pointers, the rest host arrays.
+struct KzgOpenArgs {
+    int32_t npolys, nblind, npoints, nterms;
+    const uint64_t* const* coeffs;
+    const size_t* n;
+    const uint64_t* const* blind;
+    const size_t* nb;
+    const uint64_t* points;
+    const int32_t *term_point, *term_poly, *term_blind;
+    const size_t* term_shift;
+    const uint64_t* term_coeff;
+};
+struct KzgOpenHost {
+    uint64_t* w_xy;
+    uint8_t* w_inf;
+    uint64_t* random_v;
+    uint64_t* evals;
+};
+
+// What one point needs: the linear combinations (a run of KzgLcTerm records each) and where its vectors go.
+struct KzgGroup {
+    size_t first, count, len, shift;    // terms [first, first + count) of the lc table; len = longest polynomial
+};
+struct KzgPointPlan {
+    std::vector<KzgGroup> g;            // by shift, over powers_of_g
+    KzgGroup b{0, 0, 0, 0};             // the blinding polynomials, over powers_of_gamma_g
+    size_t wlen = 0, woff = 0, boff = 0;   // witness vector length; offsets of the two vectors in the scalar buffer
+};
+
+// One batch opening enqueued on `caller` (null: the home lane's stream): per point and per distinct shift a linear
+// combination, its quotient added at the shift; the blinding combination's quotient and value; every term's
+// evaluation; into_repr of all witness vectors; the 2 x npoints MSMs in one lane acquisition; the pair sums.
+static void kzg_open_batch_impl(uint64_t handle_g, uint64_t handle_gamma_g, const KzgOpenArgs& a, int home, cudaStream_t caller,
+                                uint64_t* d_out_w, uint64_t* d_out_rv, uint64_t* d_out_evals, const KzgOpenHost* host) {
+    std::shared_ptr<BasesReg> rg = kzg_powers(handle_g, -1, "powers_of_g");
+    if (a.npoints < 0 || 2 * a.npoints > ZKM_NUM_LANES - 2) ZKM_FAIL(ZKM_ERR_ARG, "npoints must be 0..%d", (ZKM_NUM_LANES - 2) / 2);
+    if (a.npolys < 0 || a.nblind < 0 || a.nterms < 0) ZKM_FAIL(ZKM_ERR_ARG, "negative count");
+    if (a.nterms > 65535) ZKM_FAIL(ZKM_ERR_ARG, "nterms %d: at most 65535 terms per call", a.nterms);   // one grid row per term
+    if ((a.npolys && (!a.coeffs || !a.n)) || (a.nblind && (!a.blind || !a.nb)) || (a.npoints && !a.points) ||
+        (a.nterms && (!a.term_point || !a.term_poly || !a.term_blind || !a.term_shift || !a.term_coeff)))
+        ZKM_FAIL(ZKM_ERR_ARG, "null argument array");
+    const int curve = rg->curve;
+    const size_t S = (size_t)fr_words(curve), sb = S * 8;
+    std::shared_ptr<BasesReg> rh;
+    for (int i = 0; i < a.npolys; i++)
+        if (a.n[i] && !a.coeffs[i]) ZKM_FAIL(ZKM_ERR_ARG, "polynomial %d: null coefficients", i);
+    for (int i = 0; i < a.nblind; i++)
+        if (a.nb[i] && !a.blind[i]) ZKM_FAIL(ZKM_ERR_ARG, "blinding polynomial %d: null coefficients", i);
+    for (int t = 0; t < a.nterms; t++) {
+        if (a.term_point[t] < 0 || a.term_point[t] >= a.npoints) ZKM_FAIL(ZKM_ERR_ARG, "term %d: point %d out of range", t, a.term_point[t]);
+        if (a.term_poly[t] < 0 || a.term_poly[t] >= a.npolys) ZKM_FAIL(ZKM_ERR_ARG, "term %d: polynomial %d out of range", t, a.term_poly[t]);
+        if (a.term_blind[t] < -1 || a.term_blind[t] >= a.nblind) ZKM_FAIL(ZKM_ERR_ARG, "term %d: blinding polynomial %d out of range", t, a.term_blind[t]);
+        const size_t n = a.n[a.term_poly[t]], s = a.term_shift[t];
+        if (n && (s > rg->n || n - 1 > rg->n - s))
+            ZKM_FAIL(ZKM_ERR_HANDLE, "term %d: shift %zu + %zu witness coefficients exceed the %zu registered powers", t, s, n - 1, rg->n);
+        if (a.term_blind[t] >= 0) {
+            if (!rh) rh = kzg_powers(handle_gamma_g, curve, "powers_of_gamma_g");
+            const size_t k = a.nb[a.term_blind[t]];
+            if (k && k - 1 > rh->n) ZKM_FAIL(ZKM_ERR_HANDLE, "term %d: %zu hiding witness coefficients exceed powers_of_gamma_g", t, k - 1);
+        }
+    }
+    // ---- host plan: the lc table, grouped by point and shift, and the layout of every device buffer
+    std::vector<KzgPointPlan> pp(a.npoints);
+    std::vector<std::pair<size_t, int>> lc;   // (kind: 0 poly / 1 blind, index) per lc record, with its term
+    std::vector<int> lc_term;
+    size_t maxlen = 0, nscal = 0;
+    for (int i = 0; i < a.npoints; i++) {
+        KzgPointPlan& P = pp[i];
+        std::map<size_t, std::vector<int>> by_shift;
+        std::vector<int> blinds;
+        for (int t = 0; t < a.nterms; t++) {
+            if (a.term_point[t] != i) continue;
+            by_shift[a.term_shift[t]].push_back(t);
+            if (a.term_blind[t] >= 0) blinds.push_back(t);
+        }
+        for (auto& kv : by_shift) {
+            KzgGroup g{lc.size(), kv.second.size(), 0, kv.first};
+            for (int t : kv.second) {
+                lc.push_back({0, a.term_poly[t]});
+                lc_term.push_back(t);
+                g.len = std::max(g.len, a.n[a.term_poly[t]]);
+            }
+            if (g.len) P.wlen = std::max(P.wlen, g.shift + g.len - 1);
+            maxlen = std::max(maxlen, g.len);
+            P.g.push_back(g);
+        }
+        P.b = KzgGroup{lc.size(), blinds.size(), 0, 0};
+        for (int t : blinds) {
+            lc.push_back({1, a.term_blind[t]});
+            lc_term.push_back(t);
+            P.b.len = std::max(P.b.len, a.nb[a.term_blind[t]]);
+        }
+        maxlen = std::max(maxlen, P.b.len);
+        P.woff = nscal;
+        nscal += P.wlen;
+        P.boff = nscal;
+        nscal += P.b.len ? P.b.len - 1 : 0;
+    }
+    std::vector<DevItem> items(2 * a.npoints);
+    for (int i = 0; i < a.npoints; i++) {
+        items[2 * i].reg = rg;
+        items[2 * i].offset = 0;
+        items[2 * i].n = pp[i].wlen;
+        items[2 * i + 1].reg = rh ? rh : rg;
+        items[2 * i + 1].offset = 0;
+        items[2 * i + 1].n = pp[i].b.len ? pp[i].b.len - 1 : 0;
+    }
+    const KzgOps ops = kzg_ops(curve);
+    const ItemsPlan plan = plan_items(items, home);
+    MultiLaneGuard lanes(plan.devs, caller, &plan.keys);
+    Context* hc = lanes.c[0];
+    ZKM_CUDA(cudaSetDevice(hc->device));
+    if (!caller) caller = hc->stream;
+    StreamScope scope(hc, caller);
+    // input region (io_scalars): [host form: polynomials | blinding polynomials] points | lc records | eval records
+    std::vector<size_t> poff(a.npolys), bofs(a.nblind);
+    size_t in_bytes = 0;
+    if (host) {
+        for (int i = 0; i < a.npolys; i++) { poff[i] = in_bytes; in_bytes += a.n[i] * sb; }
+        for (int i = 0; i < a.nblind; i++) { bofs[i] = in_bytes; in_bytes += a.nb[i] * sb; }
+    }
+    const size_t pts_off = in_bytes, lc_off = pts_off + a.npoints * sb, ev_off = lc_off + lc.size() * sizeof(KzgLcTerm);
+    const size_t in_total = ev_off + (size_t)a.nterms * sizeof(KzgEvalTerm);
+    char* d_in = (char*)hc->io_scalars.get(in_total + 16);
+    std::vector<char> staged;      // the device form stages from pageable memory: the driver copies it before h2d returns
+    char* blob;
+    if (host) {
+        blob = (char*)hc->pin_in.get(in_total + 16);
+        for (int i = 0; i < a.npolys; i++) if (a.n[i]) memcpy(blob + poff[i], a.coeffs[i], a.n[i] * sb);
+        for (int i = 0; i < a.nblind; i++) if (a.nb[i]) memcpy(blob + bofs[i], a.blind[i], a.nb[i] * sb);
+    } else {
+        staged.resize(in_total);
+        blob = staged.data();
+        // the kernels read the polynomials in place: 16-byte aligned, in the memory of the device the call runs on
+        auto check_ptr = [&](const uint64_t* ptr, const char* what, int i) {
+            if ((uintptr_t)ptr & 15) ZKM_FAIL(ZKM_ERR_ARG, "%s %d: device pointer not 16-byte aligned", what, i);
+            if (home_device_of(ptr) != home) ZKM_FAIL(ZKM_ERR_ARG, "%s %d: not on the device of d_out_w", what, i);
+        };
+        for (int i = 0; i < a.npolys; i++)
+            if (a.n[i]) check_ptr(a.coeffs[i], "polynomial", i);
+        for (int i = 0; i < a.nblind; i++)
+            if (a.nb[i]) check_ptr(a.blind[i], "blinding polynomial", i);
+    }
+    auto poly_ptr = [&](int i) { return host ? (uint64_t)(uintptr_t)(d_in + poff[i]) : (uint64_t)(uintptr_t)a.coeffs[i]; };
+    auto blind_ptr = [&](int i) { return host ? (uint64_t)(uintptr_t)(d_in + bofs[i]) : (uint64_t)(uintptr_t)a.blind[i]; };
+    if (a.npoints) memcpy(blob + pts_off, a.points, a.npoints * sb);
+    for (size_t k = 0; k < lc.size(); k++) {
+        KzgLcTerm rec;
+        memset(&rec, 0, sizeof(rec));
+        const int t = lc_term[k], idx = lc[k].second;
+        rec.ptr = lc[k].first ? blind_ptr(idx) : poly_ptr(idx);
+        rec.n = lc[k].first ? a.nb[idx] : a.n[idx];
+        memcpy(rec.coeff, a.term_coeff + (size_t)t * S, sb);
+        memcpy(blob + lc_off + k * sizeof(KzgLcTerm), &rec, sizeof(rec));
+    }
+    uint64_t max_n = 0;
+    for (int t = 0; t < a.nterms; t++) {
+        KzgEvalTerm rec{poly_ptr(a.term_poly[t]), a.n[a.term_poly[t]], (uint64_t)a.term_point[t], 0};
+        max_n = std::max<uint64_t>(max_n, rec.n);
+        memcpy(blob + ev_off + t * sizeof(KzgEvalTerm), &rec, sizeof(rec));
+    }
+    h2d(d_in, blob, in_total, caller);
+    const uint64_t* d_pts = (const uint64_t*)(d_in + pts_off);
+    const KzgLcTerm* d_lc = (const KzgLcTerm*)(d_in + lc_off);
+    // scratch (ntt_a): the combination and its quotient; vectors (io_bases): the witness and hiding-witness scalars
+    char* scratch = (char*)hc->ntt_a.get(2 * (maxlen ? maxlen : 1) * sb);
+    uint64_t* d_p = (uint64_t*)scratch;
+    uint64_t* d_q = (uint64_t*)(scratch + (maxlen ? maxlen : 1) * sb);
+    char* d_vec = (char*)hc->io_bases.get((nscal ? nscal : 1) * sb);
+    // outputs (io_out): MSM slots | packed records | sums | random_v | evals | eval partials | tickets
+    const unsigned eblocks = kzg_eval_blocks(hc->sm_count, (uint32_t)a.nterms, max_n);
+    const size_t np = a.npoints, rb = rec_bytes(curve, 1), r1 = (rb + 15) & ~(size_t)15;
+    const size_t o_packed = 2 * np * r1, o_sums = o_packed + ((2 * np * rb + 15) & ~(size_t)15), o_rv = o_sums + np * r1;
+    const size_t o_ev = o_rv + np * sb, o_part = o_ev + a.nterms * sb, o_tick = o_part + (size_t)a.nterms * eblocks * sb;
+    char* o = (char*)hc->io_out.get(o_tick + a.nterms * 4 + 16);
+    uint64_t* rv = host ? (uint64_t*)(o + o_rv) : d_out_rv;
+    uint64_t* ev = host ? (host->evals ? (uint64_t*)(o + o_ev) : nullptr) : d_out_evals;
+    if (nscal) ZKM_CUDA(cudaMemsetAsync(d_vec, 0, nscal * sb, caller));
+    for (int i = 0; i < a.npoints; i++) {
+        const KzgPointPlan& P = pp[i];
+        const uint64_t* z = d_pts + i * S;
+        for (const KzgGroup& g : P.g) {
+            if (g.len == 0) continue;
+            ops.lincomb(hc, d_lc + g.first, (uint32_t)g.count, g.len, d_p, caller);
+            kzg_quotient_run(hc, curve, d_p, g.len, z, d_q, nullptr, caller);
+            ops.shift_add(hc, d_q, g.len - 1, (uint64_t*)(d_vec + (P.woff + g.shift) * sb), caller);
+        }
+        if (P.b.len) {   // random_v = R(z) comes with the division (the scan's value at chunk 0)
+            ops.lincomb(hc, d_lc + P.b.first, (uint32_t)P.b.count, P.b.len, d_p, caller);
+            kzg_quotient_run(hc, curve, d_p, P.b.len, z, (uint64_t*)(d_vec + P.boff * sb), rv + i * S, caller);
+        } else {
+            ZKM_CUDA(cudaMemsetAsync(rv + i * S, 0, sb, caller));
+        }
+    }
+    if (ev && a.nterms) {
+        uint32_t* tickets = (uint32_t*)(o + o_tick);
+        ZKM_CUDA(cudaMemsetAsync(tickets, 0, a.nterms * 4, caller));
+        ops.eval_many(hc, (const KzgEvalTerm*)(d_in + ev_off), (uint32_t)a.nterms, eblocks, d_pts, (uint64_t*)(o + o_part), tickets, ev,
+                      caller);
+    }
+    fr_into_repr_run(hc, curve, (const uint64_t*)d_vec, (uint64_t*)d_vec, (uint64_t)nscal, caller);   // convert_to_bigints
+    for (int i = 0; i < a.npoints; i++) {
+        items[2 * i].d_scalars = (const uint64_t*)(d_vec + pp[i].woff * sb);
+        items[2 * i].d_out = (uint64_t*)(o + 2 * i * r1);
+        items[2 * i + 1].d_scalars = (const uint64_t*)(d_vec + pp[i].boff * sb);
+        items[2 * i + 1].d_out = (uint64_t*)(o + (2 * i + 1) * r1);
+    }
+    run_items(items, plan, lanes.c.data(), caller);
+    sum_record_pairs(hc, curve, o, np, o + o_packed, o + o_sums, caller);
+    if (!host) {
+        if (np) ZKM_CUDA(cudaMemcpy2DAsync(d_out_w, rb, o + o_sums, r1, rb, np, cudaMemcpyDeviceToDevice, caller));
+        return;
+    }
+    const size_t back = (host->evals ? o_part : o_ev) - o_sums;
+    char* h = (char*)hc->pin_out.get(back + 16);
+    if (back) ZKM_CUDA(cudaMemcpyAsync(h, o + o_sums, back, cudaMemcpyDeviceToHost, caller));
+    ZKM_CUDA(cudaStreamSynchronize(caller));
+    const size_t W2 = 2 * (size_t)coord_words(curve, 1);
+    for (size_t i = 0; i < np; i++) {
+        const uint64_t* rec = (const uint64_t*)(h + i * r1);
+        memcpy(host->w_xy + i * W2, rec, W2 * 8);
+        host->w_inf[i] = rec_flag(rec[W2]);
+    }
+    if (np) memcpy(host->random_v, h + (o_rv - o_sums), np * sb);
+    if (host->evals && a.nterms) memcpy(host->evals, h + (o_ev - o_sums), a.nterms * sb);
+}
+
+int32_t zkm_kzg_commit_many(uint64_t handle_g, uint64_t handle_gamma_g, int32_t count, const uint64_t* const* coeffs,
+                            const size_t* n, const size_t* shift, const uint64_t* const* blind, const size_t* nb,
+                            uint64_t* out_xy, uint8_t* out_inf) {
+    return guarded([&] { kzg_commit_many_impl(handle_g, handle_gamma_g, count, coeffs, n, shift, blind, nb, out_xy, out_inf); });
+}
+
+int32_t zkm_kzg_open_batch(uint64_t handle_g, uint64_t handle_gamma_g, int32_t npolys, const uint64_t* const* coeffs,
+                           const size_t* n, int32_t nblind, const uint64_t* const* blind, const size_t* nb, int32_t npoints,
+                           const uint64_t* points, int32_t nterms, const int32_t* term_point, const int32_t* term_poly,
+                           const int32_t* term_blind, const size_t* term_shift, const uint64_t* term_coeff,
+                           uint64_t* out_w_xy, uint8_t* out_w_inf, uint64_t* out_random_v, uint64_t* out_evals) {
+    return guarded([&] {
+        const KzgOpenArgs a{npolys, nblind, npoints, nterms, coeffs, n, blind, nb, points, term_point, term_poly, term_blind,
+                            term_shift, term_coeff};
+        std::shared_ptr<BasesReg> rg = lookup(handle_g, 0, 0);
+        if (npoints && (!out_w_xy || !out_w_inf || !out_random_v)) ZKM_FAIL(ZKM_ERR_ARG, "null output pointer");
+        const KzgOpenHost host{out_w_xy, out_w_inf, out_random_v, out_evals};
+        kzg_open_batch_impl(handle_g, handle_gamma_g, a, rg->parts[0].dev, nullptr, nullptr, nullptr, nullptr, &host);
+    });
+}
+
+int32_t zkm_kzg_open_batch_device(uint64_t handle_g, uint64_t handle_gamma_g, int32_t npolys, const uint64_t* const* d_coeffs,
+                                  const size_t* n, int32_t nblind, const uint64_t* const* d_blind, const size_t* nb,
+                                  int32_t npoints, const uint64_t* points, int32_t nterms, const int32_t* term_point,
+                                  const int32_t* term_poly, const int32_t* term_blind, const size_t* term_shift,
+                                  const uint64_t* term_coeff, uint64_t* d_out_w, uint64_t* d_out_random_v,
+                                  uint64_t* d_out_evals, void* stream) {
+    return guarded([&] {
+        const KzgOpenArgs a{npolys, nblind, npoints, nterms, d_coeffs, n, d_blind, nb, points, term_point, term_poly, term_blind,
+                            term_shift, term_coeff};
+        lookup(handle_g, 0, 0);
+        if (!d_out_w || !d_out_random_v) ZKM_FAIL(ZKM_ERR_ARG, "null device pointer");
+        const int home = home_device_of(d_out_w);
+        kzg_open_batch_impl(handle_g, handle_gamma_g, a, home, call_stream(home, stream), d_out_w, d_out_random_v, d_out_evals, nullptr);
     });
 }
 
